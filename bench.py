@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: training ratings/s of the autoencoder hot path on synthetic data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ml10m] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ml10m] [--impl ours|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of `batch_size` rows (train.py:30: 128):
 K1 gather -> K2 encoder -> K3 decoder + masked loss + gradient -> K4 fused backward/optimizer.
@@ -74,10 +74,11 @@ def tensor_peak_tf32():
     return 1590.0 / 2.0, "fallback bf16 / 2 (B200_PROFILING.md)"
 
 
-def scoring_run(lib, m, rd, w, aux, rows, reps, warm):
+def scoring_run(lib, m, rd, w, aux, rows, reps, warm, dump_dir=None):
     """Full-catalogue scoring (train.py:239 `predict` without the mask multiply) of `rows`
     validation rows per call: device-timed with the scores left in HBM, then end to end through
-    `model.score` (host row ids in, [rows, N] float32 out)."""
+    `model.score` (host row ids in, [rows, N] float32 out). `dump_dir`: the last timed call's scores
+    go there (write_outputs)."""
     import ctypes as C
     import torch
     from omnidirectional_collaborative_filtering_b200 import _lib
@@ -118,6 +119,8 @@ def scoring_run(lib, m, rd, w, aux, rows, reps, warm):
     torch.cuda.synchronize()
     launches = lib.ocf_kernel_launches() - l0
     ms = e0.elapsed_time(e1) / reps
+    if dump_dir is not None:
+        write_outputs(dump_dir, {"scores": out.cpu().numpy()})
     lib.ocf_profile_reset()
     lib.ocf_profile_enable(1)
     run(reps)
@@ -223,6 +226,26 @@ def n_unique(a):
     """Number of distinct values (sort + compare; NumPy 2.3's hash-based np.unique is ~50x slower on these sizes)."""
     a = np.sort(np.asarray(a).ravel())
     return int(np.count_nonzero(a[1:] != a[:-1]) + 1) if a.size else 0
+
+
+DUMP_BYTES = 60 * 10 ** 6
+
+
+def write_outputs(out_dir, arrays):
+    """`arrays` (name -> float32 array) as out_dir/<name>.npy, at most DUMP_BYTES in all. Smaller arrays are written
+    whole; each array that would overrun its equal share of what is left keeps a sorted sample of its slices along
+    its longest axis, drawn with RandomState(0), so two runs at the same shapes sample the same indices."""
+    os.makedirs(out_dir, exist_ok=True)
+    left, items = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: kv[1].nbytes)
+    for k, (name, a) in enumerate(items):
+        share = left // (len(items) - k)
+        if a.nbytes > share:
+            axis = int(np.argmax(a.shape))
+            n = a.shape[axis]
+            keep = max(1, share // (a.nbytes // n))
+            a = np.take(a, np.sort(np.random.RandomState(0).choice(n, keep, replace=False)), axis=axis)
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a))
+        left -= a.nbytes
 
 
 def touched(batch, k_mask_blocks):
@@ -377,10 +400,18 @@ def main():
                     help="comma-separated workloads whose value / e2e / roofline ride along under 'other_workloads' "
                          "(default: the other four BASELINE configs when the workload is the default one; 'none' to skip)")
     ap.add_argument("--no-scoring", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, at most "
+                         "60 MB: the step's metrics and the updated weights, or the scores in --mode score); inputs are "
+                         "seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     w = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
+    if args.dump_outputs is not None and (args.impl == "reference" or world > 1):
+        ap.error("--dump-outputs covers the single-GPU path of --impl ours")
     B = args.batch_size
     cfg = {"workload": "%s-shaped synthetic (%s), rows=%s, L=%d, H=%s, %s, aux=%s, train_sparsity=%s, pass_through=%s, %s lr=%g, dropout=%s, batch_size=%d"
            % (args.workload, w["shape"], "items" if w["reverse"] else "users", w["layers"], w["hidden"], w["act"], w["aux"],
@@ -428,7 +459,7 @@ def main():
 
     if args.mode == "score":
         sampler = ClockSampler(0)
-        sc = scoring_run(lib, m, rd, w, aux, args.score_rows, K, W)
+        sc = scoring_run(lib, m, rd, w, aux, args.score_rows, K, W, args.dump_outputs)
         line = {"metric": "full-catalogue scoring rows/sec", "value": sc["value"], "unit": "rows/s", "n_gpus": 1, "steps": K,
                 "warmup": W, "ms_per_step": sc["ms_per_call"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "tf32 operands, f32 accumulate", "data": "synthetic",
@@ -483,6 +514,11 @@ def main():
     torch.cuda.synchronize()
     launches = lib.ocf_kernel_launches() - launches0
     ms = e0.elapsed_time(e1)
+    if args.dump_outputs is not None:         # before the steps below move the weights on
+        outs = {"metrics": np.array(m.wait_metrics(m.steps_logged() - 1), dtype=np.float32)}
+        for i, a in enumerate(m.get_weights()):
+            outs["%s_%d" % ("kernel" if i % 2 == 0 else "bias", i // 2)] = a
+        write_outputs(args.dump_outputs, outs)
     # the timed region lasts a few ms, nvidia-smi samples every 100 ms: keep the same steps running
     # for ~0.6 s so the clock / throttle record is taken under this load
     t_hold = time.perf_counter()

@@ -43,6 +43,34 @@ def test_step_bytes_of_shards_add_up_to_less_than_twice_the_whole():
         assert np.isclose(a0[k] + a1[k], a[k])
 
 
+def test_write_outputs_caps_the_dump_with_a_fixed_sample(tmp_path, monkeypatch):
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 20)
+    rs = np.random.RandomState(3)
+    arrays = {"metrics": rs.rand(6).astype(np.float32), "kernel_0": rs.rand(4000, 64).astype(np.float32),
+              "bias_0": rs.rand(64).astype(np.float32), "kernel_1": rs.rand(64, 3000).astype(np.float32)}
+    for run in ("a", "b"):
+        bench.write_outputs(str(tmp_path / run), arrays)
+    got = {n: np.load(str(tmp_path / "a" / (n + ".npy"))) for n in arrays}
+    assert sum(a.nbytes for a in got.values()) <= 1 << 20
+    assert np.array_equal(got["metrics"], arrays["metrics"]) and np.array_equal(got["bias_0"], arrays["bias_0"])
+    assert got["kernel_0"].shape[1] == 64 and 0 < got["kernel_0"].shape[0] < 4000
+    assert got["kernel_1"].shape[0] == 64 and 0 < got["kernel_1"].shape[1] < 3000
+    idx = [int(np.flatnonzero((arrays["kernel_0"] == r).all(axis=1))[0]) for r in got["kernel_0"]]
+    assert idx == sorted(set(idx))                                 # whole rows of the original, in order
+    for n in arrays:
+        assert got[n].dtype == np.float32 and np.array_equal(got[n], np.load(str(tmp_path / "b" / (n + ".npy"))))
+
+
+def test_bench_rejects_runs_without_timed_steps():
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", "0"], capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and "--steps" in out.stderr and out.stdout == ""
+
+
 def test_reference_arm_runs_on_rank_0_only():
     """Under torchrun the reference arm is rank 0's job: the other ranks exit 0 without work or output."""
     import os

@@ -11,6 +11,7 @@ def test_reader_plans_match_reference(golden_cases, golden_datasets, golden_batc
     for case in golden_cases:
         ds = golden_datasets[case["dataset"]]
         rd = product_reader(ds, case["eval_mode"])
+        rd.rng_on_device = False      # host stream where a GPU exists too: rng_after is read from np.random itself
         np.random.seed(case["seed"])
         if case["eval_mode"] == "ablation":
             rd.split_for_validation(case["val_split"], seed=case["split_seed"])
@@ -40,6 +41,7 @@ def test_reader_plans_match_reference(golden_cases, golden_datasets, golden_batc
 
 def test_scalar_sparsity_is_accepted(golden_datasets):
     rd = product_reader(golden_datasets["rev"], "ablation")
+    rd.rng_on_device = False          # host stream where a GPU exists too: a's flags are drawn before the reseed
     rd.split_for_validation([0.5, 0.25, 0.25], seed=1)
     np.random.seed(4)
     a = next(rd.data_gen(4, 0.4, "test"))

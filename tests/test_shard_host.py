@@ -25,6 +25,7 @@ def test_shard_batches_are_column_slices_of_the_reference(golden_cases, golden_d
         ds = golden_datasets[case["dataset"]]
         for rank in range(world):
             rd = _shard_reader(ds, case["eval_mode"], rank, world)
+            rd.rng_on_device = False  # host stream where a GPU exists too: rng_after is read from np.random itself
             lo, hi = rd.col_range
             np.random.seed(case["seed"])
             if case["eval_mode"] == "ablation":
