@@ -264,7 +264,6 @@ struct ocf_model {
   struct StepGraph { cudaGraphExec_t exec = nullptr; int kernels = 0; int seen = 0; bool failed = false; };
   std::map<std::tuple<uint64_t, int, int, int, int>, StepGraph> graphs;
   cudaStream_t cap = nullptr;     // capture stream
-  cudaStream_t cap_lo = nullptr;  // capture stream of the batch-side work list when the batch streams run at low priority (OCF_GATHER_PRIO=0)
   bool capturing = false;
   int* d_err = nullptr;
   int64_t steps_logged = 0;
@@ -275,7 +274,6 @@ struct ocf_model {
   int4* col_tasks = nullptr;
   int4* col_heavy = nullptr;      // tasks with more than HEAVY_N matches (batch-side K4a only), same capacity as col_tasks
   int* col_counters = nullptr;
-  float* gemm_part = nullptr;     // split-K partials of the hidden-layer GEMMs
   int32_t* topk_cols = nullptr;   // top-k epilogue outputs [max_rows, 512] (allocated with dense_out's arena)
   float* topk_scores = nullptr;
   size_t topk_cap = 0;
@@ -317,10 +315,6 @@ constexpr int N_REGPART = 64;
 
 // Launch with the programmatic-stream-serialization attribute (PDL, ocf_common.cuh): only for kernels that call
 // pdl_wait() before they touch memory, and only when the previous operation in the stream is a kernel.
-static bool pdl_on() {
-  static const bool on = [] { const char* e = std::getenv("OCF_NO_PDL"); return !(e && e[0] == '1'); }();
-  return on;
-}
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(bool pdl, void (*kern)(KArgs...), dim3 grid, dim3 block, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg{};
@@ -328,7 +322,7 @@ static cudaError_t launch_pdl(bool pdl, void (*kern)(KArgs...), dim3 grid, dim3 
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = (pdl && pdl_on()) ? 1 : 0;
+  cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
   return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
@@ -588,17 +582,9 @@ extern "C" int ocf_pair_destroy(ocf_pair* p) {
 // ============================================================================================
 // Upper bound of the work items of any batch within (max_rows, max_entries): pick_chunk() keeps
 // the chunk length >= ceil(entries / TARGET_ITEMS), so items <= TARGET_ITEMS + rows.
-constexpr int64_t TARGET_ITEMS_DEFAULT = 148 * 6;
-static int64_t target_items() {          // $OCF_TARGET_ITEMS: experiments with the work-item granularity
-  static const int64_t v = [] {
-    const char* e = std::getenv("OCF_TARGET_ITEMS");
-    const long long x = e ? std::atoll(e) : 0;
-    return (int64_t)(x >= 148 && x <= 148 * 64 ? x : TARGET_ITEMS_DEFAULT);
-  }();
-  return v;
-}
+constexpr int64_t TARGET_ITEMS = 148 * 6;
 static int max_items_for(int max_rows, int64_t max_entries) {
-  return (int)std::min<int64_t>(max_entries / 32 + max_rows + 1, std::max(target_items(), TARGET_ITEMS_DEFAULT) + max_rows + 1);
+  return (int)std::min<int64_t>(max_entries / 32 + max_rows + 1, TARGET_ITEMS + max_rows + 1);
 }
 
 // Fixed for the life of a batch object (sized by its capacity), so that every device pointer a kernel
@@ -639,10 +625,9 @@ extern "C" int ocf_batch_create(int32_t max_rows, int64_t max_entries, ocf_batch
   if (cudaEventCreateWithFlags(&b->copied, cudaEventDisableTiming) != cudaSuccess)
     return bail(fail(OCF_ERR_CUDA, "ocf_batch_create: event creation failed"));
   {
-    int lo = 0, hi = 0;
-    cudaDeviceGetStreamPriorityRange(&lo, &hi);
-    static const bool normal_prio = [] { const char* e = std::getenv("OCF_GATHER_PRIO"); return e && e[0] == '0'; }();
-    if (cudaStreamCreateWithPriority(&b->gstream, cudaStreamNonBlocking, normal_prio ? lo : hi) != cudaSuccess ||
+    int hi = 0;
+    cudaDeviceGetStreamPriorityRange(nullptr, &hi);
+    if (cudaStreamCreateWithPriority(&b->gstream, cudaStreamNonBlocking, hi) != cudaSuccess ||
         cudaEventCreateWithFlags(&b->gathered, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&b->wl_ready, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&b->consumed, cudaEventDisableTiming) != cudaSuccess)
@@ -689,7 +674,7 @@ extern "C" int ocf_batch_destroy(ocf_batch* b) {
 // Work items: chunks of <= CH ratings of one row, CH sized so that the row-centric kernels get
 // a few CTAs per SM whatever the batch looks like.
 static int pick_chunk(int64_t n_entries) {
-  int64_t ch = (n_entries + target_items() - 1) / target_items();
+  int64_t ch = (n_entries + TARGET_ITEMS - 1) / TARGET_ITEMS;
   ch = (int64_t)align_up((size_t)std::max<int64_t>(ch, 1), 32);
   return (int)std::max<int64_t>(ch, 32);
 }
@@ -774,13 +759,8 @@ static int launch_gather(ocf_batch* b, cudaStream_t stream) {
   return OCF_OK;
 }
 
-static bool async_gather() {          // OCF_SYNC_GATHER=1: fills run on the caller's stream, in its order
-  static const bool on = [] { const char* e = std::getenv("OCF_SYNC_GATHER"); return !(e && e[0] == '1'); }();
-  return on;
-}
 // The stream a fill of `b` runs on, ordered after the last consumer of the batch's tiles.
-static cudaStream_t fill_begin(ocf_batch* b, cudaStream_t user) {
-  if (!async_gather() || b->gstream == nullptr) return user;
+static cudaStream_t fill_begin(ocf_batch* b) {
   if (b->consumed_valid) cudaStreamWaitEvent(b->gstream, b->consumed, 0);
   return b->gstream;
 }
@@ -797,7 +777,8 @@ static int batch_acquire(const ocf_batch* b, cudaStream_t st) {
 }
 static int batch_release(const ocf_batch* cb, cudaStream_t st) {
   ocf_batch* b = const_cast<ocf_batch*>(cb);
-  if (async_gather() && b->gstream != nullptr) { OCF_CUDA(cudaEventRecord(b->consumed, st)); b->consumed_valid = true; }
+  OCF_CUDA(cudaEventRecord(b->consumed, st));
+  b->consumed_valid = true;
   return OCF_OK;
 }
 
@@ -809,7 +790,7 @@ extern "C" int ocf_batch_fill_split(ocf_batch* b, const ocf_store* store, const 
   OCF_REQUIRE(b && store && row_ids, "ocf_batch_fill_split: null argument");
   OCF_REQUIRE(keep_flags != nullptr || n_flags == 0, "ocf_batch_fill_split: null keep_flags");
   cudaStream_t user = as_stream(stream_);
-  cudaStream_t stream = fill_begin(b, user);
+  cudaStream_t stream = fill_begin(b);
   OCF_TRY(prepare_rowslot(b, store, row_ids, n_rows, stream, "ocf_batch_fill_split"));
   OCF_TRY(batch_stage(b, row_ids, n_rows, store->h_rowptr, nullptr, store->n_rows, keep_flags, n_flags, stream,
                       b->tag, pass_through ? 1 : 0, aux_var_value));
@@ -859,7 +840,7 @@ extern "C" int ocf_batch_fill_fixed(ocf_batch* b, const ocf_pair* pair, const in
                                     float aux_var_value, void* stream_) {
   OCF_REQUIRE(b && pair && row_ids, "ocf_batch_fill_fixed: null argument");
   cudaStream_t user = as_stream(stream_);
-  cudaStream_t stream = fill_begin(b, user);
+  cudaStream_t stream = fill_begin(b);
   OCF_TRY(batch_stage(b, row_ids, n_rows, pair->in->h_rowptr, &pair->tg->h_rowptr, pair->in->n_rows, nullptr, -1, stream,
                       0u, 0, aux_var_value));
   b->dev.rowslot = nullptr; b->dev.tag = 0;
@@ -875,11 +856,10 @@ extern "C" int ocf_batch_regather(ocf_batch* b, void* stream_) {
   b->rng_mode = false;            // the first gather left the flags in the device staging
   cudaStream_t user = as_stream(stream_);
   // A re-gather has no host copy to hide. On its own stream it still overlaps the previous step (Jester: 71 -> 66 us per
-  // step), but beside a step that holds NCCL collectives it costs more than it hides (2 GPUs: 785 vs 855 M ratings/s,
-  // gpurun_out/r03a-b), so a process with a communicator keeps it on the caller's stream. OCF_REGATHER_SYNC=0|1 forces.
-  static const int forced = [] { const char* e = std::getenv("OCF_REGATHER_SYNC"); return e ? (e[0] == '1' ? 1 : 0) : -1; }();
-  const bool regather_sync = forced >= 0 ? forced == 1 : g_comms_alive.load() > 0;
-  cudaStream_t stream = regather_sync ? user : fill_begin(b, user);
+  // step), but beside a step that holds NCCL collectives it costs more than it hides (2 GPUs: 785 vs 855 M ratings/s),
+  // so a process with a communicator keeps it on the caller's stream.
+  const bool regather_sync = g_comms_alive.load() > 0;
+  cudaStream_t stream = regather_sync ? user : fill_begin(b);
   if (regather_sync) OCF_TRY(batch_acquire(b, user));
   if (stream != user && b->gathered_valid) OCF_CUDA(cudaStreamWaitEvent(stream, b->gathered, 0));   // same stream: already in order
   OCF_TRY(launch_gather(b, stream));
@@ -1132,7 +1112,7 @@ extern "C" int ocf_batch_fill_split_rng(ocf_batch* b, const ocf_store* store, co
   OCF_REQUIRE(n_rows > 0 && n_rows <= b->max_rows, "ocf_batch_fill_split_rng: row count exceeds the batch capacity");
   OCF_REQUIRE((full_len != nullptr) == (store->dev.orig_pos != nullptr), "ocf_batch_fill_split_rng: full_len goes with a store that has ocf_store_set_orig_pos");
   cudaStream_t user = as_stream(stream_);
-  cudaStream_t stream = fill_begin(b, user);
+  cudaStream_t stream = fill_begin(b);
   int64_t draws = n_rows;
   for (int r = 0; r < n_rows; ++r) {
     const int32_t row = row_ids[r];
@@ -1365,7 +1345,6 @@ extern "C" int ocf_model_destroy(ocf_model* m) {
     drop_graphs(m);
     if (m->side) cudaStreamDestroy(m->side);
     if (m->cap) cudaStreamDestroy(m->cap);
-    if (m->cap_lo) cudaStreamDestroy(m->cap_lo);
     if (m->ev_fork) cudaEventDestroy(m->ev_fork);
     if (m->ev_join) cudaEventDestroy(m->ev_join);
     if (m->side2) cudaStreamDestroy(m->side2);
@@ -1634,37 +1613,6 @@ static int phase_encode(ocf_model* m, const ocf_batch* b, cudaStream_t st, float
   return OCF_OK;
 }
 
-constexpr size_t GEMM_PART_FLOATS = (size_t)8 * 512 * 1024;   // split-K scratch (16 MB), models with hidden-to-hidden layers only
-static float* g_gemm_part_of(ocf_model* m);
-
-static int launch_gemm(ocf_model* m, bool ta, bool tb, const float* A, int lda, const float* Bm, int ldb, int M, int N, int K,
-                       GemmEpi ep, cudaStream_t st) {
-  dim3 grid((N + 63) / 64, (M + 63) / 64);
-  // few output tiles and a long contraction: split K over grid.z, reduce + epilogue in a second kernel
-  int S = 1;
-  while (S < 8 && (int)(grid.x * grid.y) * S * 2 <= m->sm_count * 2 && K / (S * 2) >= 64 &&
-         (size_t)(S * 2) * M * N <= GEMM_PART_FLOATS)
-    S *= 2;
-  ep.part = nullptr;
-  if (S > 1) { ep.part = g_gemm_part_of(m); if (ep.part == nullptr) S = 1; }
-  grid.z = S;
-  if (!ta && !tb) k_sgemm<false, false><<<grid, 256, 0, st>>>(A, lda, Bm, ldb, M, N, K, ep);
-  else if (ta && !tb) k_sgemm<true, false><<<grid, 256, 0, st>>>(A, lda, Bm, ldb, M, N, K, ep);
-  else if (!ta && tb) k_sgemm<false, true><<<grid, 256, 0, st>>>(A, lda, Bm, ldb, M, N, K, ep);
-  else k_sgemm<true, true><<<grid, 256, 0, st>>>(A, lda, Bm, ldb, M, N, K, ep);
-  OCF_LAUNCHED();
-  if (S > 1) {
-    k_gemm_reduce<<<(M * ((N + 3) / 4) + 255) / 256, 256, 0, st>>>(M, N, S, ep);
-    OCF_LAUNCHED();
-  }
-  return OCF_OK;
-}
-
-static float* g_gemm_part_of(ocf_model* m) {
-  if (m->gemm_part == nullptr && !m->capturing && m->mem.get(&m->gemm_part, GEMM_PART_FLOATS) != OCF_OK) m->gemm_part = nullptr;
-  return m->gemm_part;
-}
-
 // bias + activation (+ dropout) of layer l from zsum[l]
 static int launch_act(ocf_model* m, int l, int B, bool training, const ocf_step_args* args, cudaStream_t st) {
   const int hp = m->hp[l];
@@ -1674,12 +1622,7 @@ static int launch_act(ocf_model* m, int l, int B, bool training, const ocf_step_
   return OCF_OK;
 }
 
-// ---- hidden [H1, H2] layers on the tensor cores (ocf_gemm_tc.cuh); OCF_NO_TC_HIDDEN=1 keeps the SIMT k_sgemm path ----
-static bool tc_hidden() {
-  static const bool on = [] { const char* e = std::getenv("OCF_NO_TC_HIDDEN"); return !(e && e[0] == '1'); }();
-  return on;
-}
-
+// ---- hidden [H1, H2] layers on the tensor cores (ocf_gemm_tc.cuh) ----
 // a_l = act(h_{l-1} . W_l + b_l) (+ dropout): D[n, b] = sum_k W[k, n] h[b, k]
 static int hidden_fwd_tc(ocf_model* m, int l, int B, const float* hin, const ActArgs& act, cudaStream_t st, bool pdl = false) {
   CUtensorMap ma, mb;
@@ -1688,7 +1631,7 @@ static int hidden_fwd_tc(ocf_model* m, int l, int B, const float* hin, const Act
   gtc::GemmTcArgs g{};
   g.kind = gtc::GEPI_FWD; g.a_mn = 1; g.b_mn = 0; g.actargs = act;
   g_prof.begin(8, st);
-  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l], B, m->hp[l - 1], st, 0, pdl && pdl_on() && !g_prof.on));
+  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l], B, m->hp[l - 1], st, 0, pdl && !g_prof.on));
   g_prof.end(8, st);
   return OCF_OK;
 }
@@ -1702,7 +1645,7 @@ static int hidden_dz_tc(ocf_model* m, int l, int B, bool drop, cudaStream_t st, 
   g.kind = gtc::GEPI_DZ; g.a_mn = 0; g.b_mn = 0;
   g.C = m->dz[l - 1]; g.ldc = m->hp[l - 1]; g.aux0 = m->act[l - 1]; g.aux1 = drop ? m->dscale[l - 1] : nullptr; g.act = m->cfg.activation;
   g_prof.begin(8, st);
-  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l - 1], B, m->hp[l], st, 0, pdl && pdl_on() && !g_prof.on));
+  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l - 1], B, m->hp[l], st, 0, pdl && !g_prof.on));
   g_prof.end(8, st);
   return OCF_OK;
 }
@@ -1718,7 +1661,7 @@ static int hidden_dw_tc(ocf_model* m, int l, int B, const float* hin, const OptD
   if (grad_out) { g.kind = gtc::GEPI_STORE; g.C = grad_out; }
   else { g.kind = gtc::GEPI_UPDATE; g.C = ly.W; g.s1 = ly.Ws1; g.s2 = ly.Ws2; g.opt = opt; }
   g_prof.begin(8, st);
-  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l], m->hp[l - 1], B, st, 0, pdl && pdl_on() && !g_prof.on));
+  OCF_TRY(gtc::launch(ma, mb, g, m->hp[l], m->hp[l - 1], B, st, 0, pdl && !g_prof.on));
   g_prof.end(8, st);
   return OCF_OK;
 }
@@ -1728,12 +1671,8 @@ static int hidden_dw_tc(ocf_model* m, int l, int B, const float* hin, const OptD
 // into the exchange).
 // after_kernel: the previous operation in the stream is a kernel (the phase's first launch may be a dependent launch)
 // An unsharded model's K3 leaves dz of the top hidden layer itself (DzFuse): dL/dh of a row is complete on this device.
-// A column shard all-reduces dL/dh first and keeps the separate kernel. OCF_OVERLAP bit 4 off: separate kernel everywhere.
-static int overlap_bits() {
-  static const int bits = [] { const char* e = std::getenv("OCF_OVERLAP"); return e ? std::atoi(e) : 7; }();
-  return bits;
-}
-static bool fuse_dz(const ocf_model* m) { return (overlap_bits() & 4) && !m->cfg.sharded && m->par_mode == 0; }
+// A column shard all-reduces dL/dh first and keeps the separate kernel.
+static bool fuse_dz(const ocf_model* m) { return !m->cfg.sharded && m->par_mode == 0; }
 
 static int phase_decode(ocf_model* m, const ocf_batch* b, bool training, const ocf_step_args* args,
                         float* dense_out, cudaStream_t st, bool act0_done = false, bool after_kernel = false) {
@@ -1744,10 +1683,8 @@ static int phase_decode(ocf_model* m, const ocf_batch* b, bool training, const o
   if (!act0_done) { OCF_TRY(launch_act(m, 0, B, training, args, st)); dep = !g_prof.on; }
   for (int l = 1; l < L; ++l) {
     // hidden layer: product + bias + activation + dropout in the GEMM's epilogue
-    GemmEpi ep{}; ep.kind = EPI_BIAS_ACT; ep.C = m->zsum[l]; ep.ldc = m->hp[l]; ep.actargs = act_args(m, l, B, training, args);
     const float* hin = drop ? m->h[l - 1] : m->act[l - 1];
-    if (tc_hidden()) OCF_TRY(hidden_fwd_tc(m, l, B, hin, ep.actargs, st, dep));
-    else OCF_TRY(launch_gemm(m, false, false, hin, m->hp[l - 1], m->layers[l].W, m->hp[l], B, m->hp[l], m->hp[l - 1], ep, st));
+    OCF_TRY(hidden_fwd_tc(m, l, B, hin, act_args(m, l, B, training, args), st, dep));
     dep = !g_prof.on;
   }
   const float* htop = drop ? m->h[L - 1] : m->act[L - 1];
@@ -1838,14 +1775,10 @@ static int launch_row_update(int hp, int kind, int sm_count, bool wide, bool hea
   return OCF_OK;
 }
 
-static bool heavy_rows() {            // OCF_NO_HEAVY=1: every update task is one warp's, whatever its length
-  static const bool on = [] { const char* e = std::getenv("OCF_NO_HEAVY"); return !(e && e[0] == '1'); }();
-  return on;
-}
 // Catalogues whose weights are within reach of the 126 MB L2 (n_cols x hp <= 32 M floats): the update is bound by its
 // longest chain of dependent L2 round trips, so long chains are split over a CTA; beyond that it is HBM-bound.
 static bool heavy_model(const ocf_model* m) {
-  return heavy_rows() && (size_t)m->cfg.n_cols * (size_t)std::max(m->hp[0], m->hp[m->L - 1]) <= ((size_t)32 << 20);
+  return (size_t)m->cfg.n_cols * (size_t)std::max(m->hp[0], m->hp[m->L - 1]) <= ((size_t)32 << 20);
 }
 
 // The model's own work list (filled inside the step).
@@ -1894,8 +1827,6 @@ static int launch_scan(ocf_model* m, const ocf_batch* b, int do_dec, int do_enc,
     a.colinfo = wl.info; a.bits = wl.bits; a.W = W; a.counters = wl.counters;
     a.matches = wl.matches; a.tasks = wl.tasks; a.colseg = wl.seg; a.heavy = heavy_model(m) ? wl.heavy : nullptr;
     a.n_cols = m->cfg.n_cols; a.nblk = m->nblk; a.bits3 = m->bits; a.dense = dense; a.do_dec = do_dec; a.do_enc = do_enc;
-    static const bool dec_first = [] { const char* e = std::getenv("OCF_DEC_FIRST"); return !(e && e[0] == '0'); }();
-    a.dec_first = dec_first ? 1 : 0;
     const int grid = item_grid(m, b);
     g_prof.begin(3, st);
     k_sort_count<<<grid, 128, 0, st>>>(a);
@@ -1948,8 +1879,6 @@ static int launch_rows(ocf_model* m, const ocf_batch* b, int do_dec, int do_enc,
   r.Wenc = enc.W; r.We_s1 = enc.Ws1; r.We_s2 = enc.Ws2;
   r.n_cols = m->cfg.n_cols; r.bits = m->bits; r.bt_hdr = b->dev.hdr; r.opt = opt;
   r.task_cap = m->cfg.n_cols * (m->nblk + 1);
-  static const bool k4b_stream = [] { const char* e = std::getenv("OCF_K4B_STREAM"); return !(e && e[0] == '0'); }();
-  r.stream = k4b_stream ? 1 : 0;
   r.dense = grad_mode ? 0 : opt.dense; r.n_arr = 0; r.only = only;
   if (grad_mode) { r.Gdec = m->gW[L]; r.Genc = m->gW[0]; r.gbdec = m->gb[L]; }
   if (do_dec) r.arr_map[r.n_arr++] = 0;
@@ -1997,18 +1926,16 @@ static int phase_update(ocf_model* m, const ocf_batch* b, const ocf_step_args* a
   const int hpd = m->hp[L - 1], hpe = m->hp[0];
   // What is not on the critical path K3 -> (backward products of the hidden layers) -> encoder rows runs on a second
   // stream beside it and joins at the end of the step:
-  //   bit 4  the bias gradients (column sums of dz; K3 has already left dz of the top layer, fuse_dz) and, riding along
-  //          with the first of them, the step's metric record;
-  //   bit 1  the gradient product + update of hidden layer l: needs dz_l, and W_l no longer being read by the backward product;
-  //   bit 2  the decoder rows' update: needs nothing after K3 (only when it is a real kernel: a catalogue of a few
-  //          hundred columns updates in one small launch either way).
-  // OCF_OVERLAP=<bits> (default 7), 0: one stream, separate dz kernel.
-  const int bits = overlap_bits();
+  //   * the bias gradients (column sums of dz; K3 has already left dz of the top layer, fuse_dz) and, riding along
+  //     with the first of them, the step's metric record;
+  //   * the gradient product + update of hidden layer l: needs dz_l, and W_l no longer being read by the backward product;
+  //   * the decoder rows' update: needs nothing after K3 (only when it is a real kernel: a catalogue of a few
+  //     hundred columns updates in one small launch either way).
   const bool fz = fuse_dz(m) && !grad_mode;
   const bool side_ok = !grad_mode && m->par_mode == 0 && wl_current(m, b) && m->side2 != nullptr && !g_prof.on;
   const bool side_bias = side_ok && fz;
-  const bool split_dw = side_ok && L > 1 && tc_hidden() && (bits & 1);
-  const bool split = side_ok && L > 1 && (bits & 2) && (size_t)m->cfg.n_cols * (size_t)hpd >= ((size_t)1 << 20);
+  const bool split_dw = side_ok && L > 1;
+  const bool split = side_ok && L > 1 && (size_t)m->cfg.n_cols * (size_t)hpd >= ((size_t)1 << 20);
   bool forked = false;
   if (side_bias || (split && dec.trainable)) {
     OCF_CUDA(cudaEventRecord(m->ev_fork2, st));
@@ -2036,10 +1963,7 @@ static int phase_update(ocf_model* m, const ocf_batch* b, const ocf_step_args* a
   for (int l = L - 1; l >= 1; --l) {
     Layer& ly = m->layers[l];
     // dz_{l-1} = (dz_l . W_l^T) * dropout scale * act'(a_{l-1})   (uses W_l before its update)
-    GemmEpi ep{}; ep.kind = EPI_DZ; ep.C = m->dz[l - 1]; ep.ldc = m->hp[l - 1]; ep.aux0 = m->act[l - 1];
-    ep.aux1 = drop ? m->dscale[l - 1] : nullptr; ep.act = m->cfg.activation;
-    if (tc_hidden()) OCF_TRY(hidden_dz_tc(m, l, B, drop, st, dep));
-    else OCF_TRY(launch_gemm(m, false, true, m->dz[l], m->hp[l], ly.W, m->hp[l], B, m->hp[l - 1], m->hp[l], ep, st));
+    OCF_TRY(hidden_dz_tc(m, l, B, drop, st, dep));
     dep = !g_prof.on;
     const bool to_side = side_bias || (split_dw && ly.trainable);
     if (to_side) {
@@ -2055,11 +1979,8 @@ static int phase_update(ocf_model* m, const ocf_batch* b, const ocf_step_args* a
     OCF_LAUNCHED();
     if (ly.trainable) {
       // dW_l = h_{l-1}^T . dz_l, fused with the update of W_l
-      GemmEpi eu{}; eu.kind = EPI_UPDATE; eu.C = ly.W; eu.ldc = m->hp[l]; eu.s1 = ly.Ws1; eu.s2 = ly.Ws2; eu.opt = opt;
-      if (grad_mode) { eu.kind = EPI_STORE; eu.C = m->gW[l]; }
       const float* hin = drop ? m->h[l - 1] : m->act[l - 1];
-      if (tc_hidden()) OCF_TRY(hidden_dw_tc(m, l, B, hin, opt, grad_mode ? m->gW[l] : nullptr, split_dw ? m->side2 : st, split_dw ? side_bias : dep));
-      else OCF_TRY(launch_gemm(m, true, false, hin, m->hp[l - 1], m->dz[l], m->hp[l], m->hp[l - 1], m->hp[l], B, eu, st));
+      OCF_TRY(hidden_dw_tc(m, l, B, hin, opt, grad_mode ? m->gW[l] : nullptr, split_dw ? m->side2 : st, split_dw ? side_bias : dep));
     }
   }
   // catalogue-wide kernels: encoder rows and decoder rows of every touched column
@@ -2254,22 +2175,13 @@ static int eval_body(ocf_model* m, ocf_batch* b, const ocf_step_args* args, cuda
   return launch_metrics(m, b->dev.B, args, n_reg, false, st);
 }
 
-static bool graphs_enabled() {
-  static const bool on = [] { const char* e = std::getenv("OCF_NO_GRAPH"); return !(e && e[0] == '1'); }();
-  return on;
-}
-
 // ---- K4a ahead of the step --------------------------------------------------------------------------
 // The column grouping needs nothing but the gathered batch, so a single-GPU training step runs it on the batch's
 // own stream right behind the gather: it executes under whatever step the device is still busy with (the host
-// enqueues a step or two ahead) instead of beside this step's K2 / K3. OCF_NO_AHEAD=1: back inside the step.
-static bool ahead_enabled() {
-  static const bool on = [] { const char* e = std::getenv("OCF_NO_AHEAD"); return !(e && e[0] == '1'); }();
-  return on;
-}
+// enqueues a step or two ahead) instead of beside this step's K2 / K3.
 static bool ahead_ok(const ocf_model* m, const ocf_batch* b, const ocf_step_args* args) {
-  return ahead_enabled() && m->par_mode == 0 && m->comm == nullptr && (args == nullptr || args->phase == 0) && b->mode == 1 &&
-         b->store != nullptr && !b->store->has_dups && b->gstream != nullptr && b->gathered_valid &&
+  return m->par_mode == 0 && m->comm == nullptr && (args == nullptr || args->phase == 0) && b->mode == 1 &&
+         b->store != nullptr && !b->store->has_dups && b->gathered_valid &&
          (m->layers[0].trainable || m->layers[m->L].trainable) && b->dev.B <= b->max_rows;
 }
 
@@ -2323,7 +2235,7 @@ static int prepare_worklist(ocf_model* m, ocf_batch* b, cudaStream_t user) {
   cudaStream_t gs = b->gstream;                                                        // the fill ran here: in order behind it
   if (b->consumed_valid) OCF_CUDA(cudaStreamWaitEvent(gs, b->consumed, 0));            // the list's previous reader
   bool done = false;
-  if (graphs_enabled() && !g_prof.on) {
+  if (!g_prof.on) {
     if (b->wl_graph != nullptr && !(b->wl_graph_sig == sig)) { cudaGraphExecDestroy(b->wl_graph); b->wl_graph = nullptr; b->wl_graph_failed = false; }
     if (b->wl_graph == nullptr && !b->wl_graph_failed) {
       const long long launched = g_launches.load();
@@ -2331,21 +2243,11 @@ static int prepare_worklist(ocf_model* m, ocf_batch* b, cudaStream_t user) {
       m->capturing = true;                         // grids sized to the batch object's capacity (item_grid)
       cudaGraph_t graph = nullptr;
       int rc = OCF_OK;
-      // captured kernel nodes inherit the capture stream's priority: the list's kernels follow the batch streams'
-      static const bool low_prio = [] { const char* e = std::getenv("OCF_GATHER_PRIO"); return e && e[0] == '0'; }();
-      cudaStream_t cs = m->cap;
-      if (low_prio) {
-        if (m->cap_lo == nullptr) {
-          int lo = 0, hi = 0;
-          cudaDeviceGetStreamPriorityRange(&lo, &hi);
-          if (cudaStreamCreateWithPriority(&m->cap_lo, cudaStreamNonBlocking, lo) != cudaSuccess) { cudaGetLastError(); m->cap_lo = nullptr; }
-        }
-        if (m->cap_lo != nullptr) cs = m->cap_lo;
-      }
-      if (cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); rc = OCF_ERR_CUDA; }
+      // captured kernel nodes inherit the capture stream's priority: m->cap runs at the batch streams' (the highest)
+      if (cudaStreamBeginCapture(m->cap, cudaStreamCaptureModeThreadLocal) != cudaSuccess) { cudaGetLastError(); rc = OCF_ERR_CUDA; }
       else {
-        rc = worklist_enqueue(m, b, sig, cs);
-        if (cudaStreamEndCapture(cs, &graph) != cudaSuccess) { cudaGetLastError(); rc = OCF_ERR_CUDA; graph = nullptr; }
+        rc = worklist_enqueue(m, b, sig, m->cap);
+        if (cudaStreamEndCapture(m->cap, &graph) != cudaSuccess) { cudaGetLastError(); rc = OCF_ERR_CUDA; graph = nullptr; }
       }
       m->capturing = was_capturing;
       b->wl_graph_kernels = (int)(g_launches.load() - launched);
@@ -2374,7 +2276,7 @@ static int run_step(ocf_model* m, ocf_batch* b, const ocf_step_args* args, bool 
   OCF_TRY(sync_step_state(m, args, st));
   auto body = [&](cudaStream_t s) { return train ? train_body(m, b, args, s) : eval_body(m, b, args, s); };
   bool done = false;
-  if (graphs_enabled() && !g_prof.on && !b->store->has_dups) {
+  if (!g_prof.on && !b->store->has_dups) {
     const auto key = std::make_tuple(b->uid, b->dev.B, train ? (wl_current(m, b) ? 3 : 1) : 0, args ? args->rows_total : 0, args ? args->row0 : 0);
     ocf_model::StepGraph& g = m->graphs[key];
     if (g.exec == nullptr && !g.failed && g.seen++ >= 1) {
@@ -2553,42 +2455,29 @@ static int ocf_score_impl(ocf_model* m, ocf_batch* b, float* out, int out_is_dev
   bool act0 = false;
   OCF_TRY(encode_for_output(m, b, st, &act0));
   if (!act0) OCF_TRY(launch_act(m, 0, B, false, nullptr, st));
-  for (int l = 1; l < L; ++l) {
-    if (tc_hidden()) { OCF_TRY(hidden_fwd_tc(m, l, B, m->act[l - 1], act_args(m, l, B, false, nullptr), st)); continue; }
-    GemmEpi ep{}; ep.kind = EPI_STORE; ep.C = m->zsum[l]; ep.ldc = m->hp[l];
-    OCF_TRY(launch_gemm(m, false, false, m->act[l - 1], m->hp[l - 1], m->layers[l].W, m->hp[l], B, m->hp[l], m->hp[l - 1], ep, st));
-    OCF_TRY(launch_act(m, l, B, false, nullptr, st));
-  }
+  for (int l = 1; l < L; ++l) OCF_TRY(hidden_fwd_tc(m, l, B, m->act[l - 1], act_args(m, l, B, false, nullptr), st));
   float* dst = out;
   if (!out_is_device) { OCF_TRY(ensure_dense(m)); dst = m->dense_out; }
   // decoder GEMM on the tensor cores: tcgen05.mma kind::tf32, accumulators in TMEM (ocf_score_tc.cuh)
   const Layer& dec = m->layers[L];
   const int hpt = m->hp[L - 1];
-  static const bool trunc = std::getenv("OCF_TC_TRUNCATE") != nullptr;   // diagnostic: let the MMA truncate fp32 -> tf32
-  static const bool single = std::getenv("OCF_TC_1CTA") != nullptr;     // diagnostic: the one-SM kernel instead of CTA pairs
   if (!m->map_w_ok) {
-    OCF_TRY(tc::make_map(&m->map_w, dec.W, hpt, (long long)align_up((size_t)m->cfg.n_cols, 2 * tc::TILE_M), tc::TILE_M, !trunc));
+    OCF_TRY(tc::make_map(&m->map_w, dec.W, hpt, (long long)align_up((size_t)m->cfg.n_cols, 2 * tc::TILE_M), tc::TILE_M));
     m->map_w_ok = true;
   }
   const int nb = tc::chunk_rows(B);
-  const int box = single ? nb : nb / 2;           // a CTA of a pair loads half of the batch-row operand
+  const int box = nb / 2;                         // a CTA of a pair loads half of the batch-row operand
   if (!m->map_h_ok || m->map_h_box != box) {
-    OCF_TRY(tc::make_map(&m->map_h, m->act[L - 1], hpt, m->act_rows, box, !trunc));
+    OCF_TRY(tc::make_map(&m->map_h, m->act[L - 1], hpt, m->act_rows, box));
     m->map_h_ok = true; m->map_h_box = box;
   }
   tc::ScoreArgs sa{};
   sa.bias = dec.b; sa.out = dst; sa.ldo = m->cfg.n_cols; sa.n_cols = m->cfg.n_cols; sa.n_rows = B;
   sa.num_k = hpt / tc::BLOCK_K; sa.n_mtiles = (m->cfg.n_cols + tc::TILE_M - 1) / tc::TILE_M; sa.n_chunks = (B + nb - 1) / nb;
   g_prof.begin(4, st);
-  if (single) {
-    if (nb == 64) OCF_TRY(tc::launch_score_nb<64>(m->map_w, m->map_h, sa, m->sm_count, st));
-    else if (nb == 128) OCF_TRY(tc::launch_score_nb<128>(m->map_w, m->map_h, sa, m->sm_count, st));
-    else OCF_TRY(tc::launch_score_nb<256>(m->map_w, m->map_h, sa, m->sm_count, st));
-  } else {
-    if (nb == 64) OCF_TRY(tc::launch_score_pair_nb<64>(m->map_w, m->map_h, sa, m->sm_count, st));
-    else if (nb == 128) OCF_TRY(tc::launch_score_pair_nb<128>(m->map_w, m->map_h, sa, m->sm_count, st));
-    else OCF_TRY(tc::launch_score_pair_nb<256>(m->map_w, m->map_h, sa, m->sm_count, st));
-  }
+  if (nb == 64) OCF_TRY(tc::launch_score_pair_nb<64>(m->map_w, m->map_h, sa, m->sm_count, st));
+  else if (nb == 128) OCF_TRY(tc::launch_score_pair_nb<128>(m->map_w, m->map_h, sa, m->sm_count, st));
+  else OCF_TRY(tc::launch_score_pair_nb<256>(m->map_w, m->map_h, sa, m->sm_count, st));
   g_prof.end(4, st);
   if (!out_is_device) {
     OCF_CUDA(cudaMemcpyAsync(out, dst, sizeof(float) * (size_t)B * m->cfg.n_cols, cudaMemcpyDeviceToHost, st));

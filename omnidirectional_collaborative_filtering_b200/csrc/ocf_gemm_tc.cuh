@@ -59,7 +59,7 @@ struct GemmTcArgs {
   int split;             // CTAs of a cluster along the contraction (gridDim.z)
   int m_valid;           // rows of the output that exist (the rest of the last tile is skipped)
   int n_valid;           // columns of the output that exist (batch rows for FWD / DZ, fan-in rows for UPDATE)
-  int terms;             // 3: hi*hi + hi*lo + lo*hi (default); 1: plain tf32 (diagnostic)
+  int terms;             // 3 (or 0): hi*hi + hi*lo + lo*hi; 1: plain tf32 (diagnostic)
   float* C; int ldc;     // DZ: dz' [b, ldc]; UPDATE / STORE: W [k, ldc]; RAW: out [col, ldc]
   const float* aux0;     // DZ: activations a [b, ldc]
   const float* aux1;     // DZ: dropout scale [b, ldc] or null
@@ -464,17 +464,12 @@ inline int launch(const CUtensorMap& ma, const CUtensorMap& mb, GemmTcArgs g, in
   }
   const int mt = (m_len + GM - 1) / GM, nt = (n_len + NB - 1) / NB;
   const int kb = (k_len + BK - 1) / BK;
-  static const int force_split = [] { const char* e = std::getenv("OCF_TC_SPLIT"); return e ? std::atoi(e) : 0; }();
   int split = pick_split(kb, mt * nt);
-  if (force_split >= 1 && force_split <= MAX_SPLIT && kb % force_split == 0) split = force_split;
   if (want_split >= 1 && want_split <= MAX_SPLIT) { split = want_split; while (kb % split) split /= 2; }
   g.split = split;
   g.k_blocks = kb / split;
   g.m_valid = m_len; g.n_valid = n_len;
-  if (g.terms == 0) {
-    static const int terms = [] { const char* e = std::getenv("OCF_TC_TERMS"); return (e && e[0] == '1') ? 1 : 3; }();
-    g.terms = terms;
-  }
+  if (g.terms == 0) g.terms = 3;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3((unsigned)mt, (unsigned)nt, (unsigned)split);
   cfg.blockDim = dim3(NTHREADS, 1, 1);

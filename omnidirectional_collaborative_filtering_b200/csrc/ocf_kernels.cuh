@@ -704,7 +704,7 @@ k_dec_fwd(BatchDev bt, const float* __restrict__ WdecT, const float* __restrict_
 // round-robin and their partial column sums are added in warp order. The launch may carry one
 // CTA more than there are unit groups: it writes the step's metric record (saves a launch on the
 // critical path of a training step).
-// dh_is_dz: the input already is dz (produced by the EPI_DZ GEMM epilogue).
+// dh_is_dz: the input already is dz (left by K3's DzFuse or by the backward product's GEPI_DZ epilogue).
 constexpr int LOG_CAP = 4096;             // steps the metric log holds
 constexpr int LOG_W = OCF_N_METRICS;
 
@@ -758,135 +758,6 @@ k_dz_bias(const float* __restrict__ dh, const float* __restrict__ a, const float
     if (s1) s1[u] = t1;
     if (s2) s2[u] = t2;
   }
-}
-
-// ============================================================================================
-// Dense GEMM for the hidden HxH layers and the SIMT scoring path (fp32, 64x64x16 tiles).
-//   C[M,N] = A'[M,K] * B'[K,N],  A'(m,k) = TA ? A[k*lda+m] : A[m*lda+k],
-//                                B'(k,n) = TB ? B[n*ldb+k] : B[k*ldb+n]
-// ============================================================================================
-enum { EPI_STORE = 0, EPI_DZ = 1, EPI_UPDATE = 2, EPI_BIAS_COL = 3, EPI_BIAS_ACT = 4 };
-
-struct GemmEpi {
-  int kind;
-  float* part;         // split-K: raw partial products [gridDim.z][M][N] (the epilogue runs in k_gemm_reduce)
-  float* C; int ldc;
-  const float* aux0;   // EPI_DZ: activation a [M, ldc];   EPI_BIAS_COL: bias [N]
-  const float* aux1;   // EPI_DZ: dropout scale or null
-  float* s1; float* s2;  // EPI_UPDATE: optimizer state, same layout as C (C = the weight)
-  int act;
-  OptDev opt;
-  ActArgs actargs;     // EPI_BIAS_ACT: bias + activation + dropout of a hidden layer's forward product (N = its padded width)
-};
-
-// One output element group (4 consecutive columns of one row) through the GEMM's epilogue.
-__device__ __forceinline__ void gemm_epilogue4(const GemmEpi& ep, const float lr, int gm, int gn, int ncols, const float v[4]) {
-  if (ep.kind == EPI_BIAS_ACT) {            // ncols == 4 always: the width is padded to 128
-    bias_act_elem(ep.actargs, gm * ep.actargs.hp4 + (gn >> 2), make_float4(v[0], v[1], v[2], v[3]));
-    return;
-  }
-  for (int j = 0; j < ncols; ++j) {
-    const size_t k = (size_t)gm * ep.ldc + gn + j;
-    float x = v[j];
-    switch (ep.kind) {
-      case EPI_STORE: ep.C[k] = x; break;
-      case EPI_DZ:
-        if (ep.aux1 != nullptr) x *= ep.aux1[k];
-        ep.C[k] = x * act_bwd(ep.act, ep.aux0[k]);
-        break;
-      case EPI_UPDATE: {
-        float w = ep.C[k], t1 = ep.s1 ? ep.s1[k] : 0.f, t2 = ep.s2 ? ep.s2[k] : 0.f;
-        opt_apply(ep.opt, lr, x, w, t1, t2);
-        ep.C[k] = w;
-        if (ep.s1) ep.s1[k] = t1;
-        if (ep.s2) ep.s2[k] = t2;
-      } break;
-      default: ep.C[k] = x + ep.aux0[gn + j]; break;
-    }
-  }
-}
-
-template <bool TA, bool TB>
-__global__ void __launch_bounds__(256)
-k_sgemm(const float* __restrict__ A, int lda, const float* __restrict__ Bm, int ldb,
-        int M, int N, int K, GemmEpi ep) {
-  __shared__ float As[16][64 + 4];
-  __shared__ float Bs[16][64 + 4];
-  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
-  const int m0 = blockIdx.y * 64, n0 = blockIdx.x * 64;
-  float acc[4][4];
-#pragma unroll
-  for (int i = 0; i < 4; ++i)
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-  // split-K: slice blockIdx.z of the contraction (a batch of 128 rows gives a 2 x 8 grid of output
-  // tiles and a 64-step K loop otherwise: latency-bound on 16 CTAs)
-  const int kchunk = ((K + (int)gridDim.z - 1) / (int)gridDim.z + 15) / 16 * 16;
-  const int kbeg = blockIdx.z * kchunk;
-  K = min(K, kbeg + kchunk);
-  for (int k0 = kbeg; k0 < K; k0 += 16) {
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-      const int e = tid + r * 256;
-      int kk, mm;
-      if (TA) { mm = e & 63; kk = e >> 6; } else { kk = e & 15; mm = e >> 4; }
-      const int gm = m0 + mm, gk = k0 + kk;
-      float va = 0.f;
-      if (gm < M && gk < K) va = TA ? A[(size_t)gk * lda + gm] : A[(size_t)gm * lda + gk];
-      As[kk][mm] = va;
-      int kb, nn;
-      if (TB) { kb = e & 15; nn = e >> 4; } else { nn = e & 63; kb = e >> 6; }
-      const int gn = n0 + nn, gkb = k0 + kb;
-      float vb = 0.f;
-      if (gn < N && gkb < K) vb = TB ? Bm[(size_t)gn * ldb + gkb] : Bm[(size_t)gkb * ldb + gn];
-      Bs[kb][nn] = vb;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int kk = 0; kk < 16; ++kk) {
-      float a[4], b[4];
-#pragma unroll
-      for (int i = 0; i < 4; ++i) { a[i] = As[kk][ty * 4 + i]; b[i] = Bs[kk][tx * 4 + i]; }
-#pragma unroll
-      for (int i = 0; i < 4; ++i)
-#pragma unroll
-        for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
-    }
-    __syncthreads();
-  }
-  const float lr = ep.kind == EPI_UPDATE ? ep.opt.st->lr : 0.f;
-#pragma unroll
-  for (int i = 0; i < 4; ++i) {
-    const int gm = m0 + ty * 4 + i;
-    if (gm >= M) continue;
-    const int gn = n0 + tx * 4;
-    if (gn >= N) continue;
-    const int ncols = min(4, N - gn);
-    if (gridDim.z > 1) {
-      for (int j = 0; j < ncols; ++j) ep.part[((size_t)blockIdx.z * M + gm) * N + gn + j] = acc[i][j];
-      continue;
-    }
-    gemm_epilogue4(ep, lr, gm, gn, ncols, acc[i]);
-  }
-}
-
-// Sum of the split-K partials in slice order + the GEMM's epilogue.
-__global__ void __launch_bounds__(256)
-k_gemm_reduce(int M, int N, int S, GemmEpi ep) {
-  const int n4 = (N + 3) / 4;
-  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= M * n4) return;
-  const int gm = idx / n4, gn = (idx - gm * n4) * 4;
-  const int ncols = min(4, N - gn);
-  const float lr = ep.kind == EPI_UPDATE ? ep.opt.st->lr : 0.f;
-  float v[4] = {0.f, 0.f, 0.f, 0.f};
-  for (int j = 0; j < ncols; ++j) {
-    const size_t e = (size_t)gm * N + gn + j;
-    float x = ep.part[e];
-    for (int z = 1; z < S; ++z) x += ep.part[(size_t)z * M * N + e];
-    v[j] = x;
-  }
-  gemm_epilogue4(ep, lr, gm, gn, ncols, v);
 }
 
 // ============================================================================================
@@ -1109,7 +980,6 @@ struct SortArgs {
   uint32_t* matches; int4* tasks; int2* colseg;
   int4* heavy;                              // (column, array, first match, matches) of every task with more than HEAVY_N matches (null: none recorded)
   int n_cols; int nblk; int3 bits3; int dense; int do_dec; int do_enc;
-  int dec_first;                            // decoder tasks fill the task array from the front, encoder tasks from the back
 };
 
 __global__ void __launch_bounds__(128) k_sort_count(SortArgs a) {
@@ -1152,9 +1022,9 @@ __global__ void __launch_bounds__(256) k_sort_alloc(SortArgs a) {
     }
   }
   if (__ballot_sync(FULL, n > 0) == 0u) return;
-  // decoder tasks (array 0, always first in arr[]) and encoder tasks are placed apart when dec_first: K4b then walks
-  // the decoder rows first, while the rows K3 has just read are still in L2
-  const int n_front = a.dec_first ? ((n_tasks > 0 && arr[0] == 0) ? 1 : 0) : n_tasks;
+  // decoder tasks (array 0, always first in arr[]) fill the task array from the front, encoder tasks from the back:
+  // K4b then walks the decoder rows first, while the rows K3 has just read are still in L2
+  const int n_front = (n_tasks > 0 && arr[0] == 0) ? 1 : 0;
   const int n_back = n_tasks - n_front;
   int sn = n, stk = n_front, ste = n_back;   // inclusive prefixes over the lanes
 #pragma unroll
@@ -1215,7 +1085,6 @@ struct RowArgs {
   int n_cols; int3 bits; const BatchHdr* bt_hdr;
   int dense; int n_arr; int arr_map[4];
   const int4* heavy;                        // tasks with more than HEAVY_N matches, walked by whole CTAs (null: every task is a warp's)
-  int stream;                               // lean variant: optimizer state loads and all row stores as evict-first traffic (OCF_K4B_STREAM=0: plain)
   int task_cap;                             // capacity of the task array: task t >= counters[1] is tasks[task_cap - 1 - (t - counters[1])] (K4a puts the encoder tasks there)
   int only;                                 // task list shared by two launches (decoder and encoder rows of different widths): 1 = decoder tasks only, 2 = encoder tasks only
   OptDev opt;
@@ -1253,7 +1122,7 @@ k_row_update(RowArgs a) {
 #pragma unroll
     for (int v = 0; v < NV; ++v) {
       w[v] = LOAD_W ? *reinterpret_cast<const float4*>(Wrow + v * 128) : make_float4(0.f, 0.f, 0.f, 0.f);
-      if (STREAM && a.stream) {
+      if (STREAM) {
         t1[v] = KIND != OCF_OPT_SGD ? __ldcs(reinterpret_cast<const float4*>(S1row + r + lane * 4 + v * 128)) : make_float4(0.f, 0.f, 0.f, 0.f);
         t2[v] = KIND == OCF_OPT_ADAM ? __ldcs(reinterpret_cast<const float4*>(S2row + r + lane * 4 + v * 128)) : make_float4(0.f, 0.f, 0.f, 0.f);
       } else {
@@ -1322,7 +1191,7 @@ k_row_update(RowArgs a) {
       opt_apply_k<KIND>(a.opt, lr, g[v].y, w[v].y, t1[v].y, t2[v].y);
       opt_apply_k<KIND>(a.opt, lr, g[v].z, w[v].z, t1[v].z, t2[v].z);
       opt_apply_k<KIND>(a.opt, lr, g[v].w, w[v].w, t1[v].w, t2[v].w);
-      if (STREAM && a.stream) {
+      if (STREAM) {
         __stcs(reinterpret_cast<float4*>(Wrow + v * 128), w[v]);
         if (KIND != OCF_OPT_SGD) __stcs(reinterpret_cast<float4*>(S1row + r + lane * 4 + v * 128), t1[v]);
         if (KIND == OCF_OPT_ADAM) __stcs(reinterpret_cast<float4*>(S2row + r + lane * 4 + v * 128), t2[v]);

@@ -11,7 +11,7 @@
 // Warp roles (320 threads): warp 0 = TMA producer (one elected lane), warp 1 = TMEM owner + MMA
 // issuer (one elected lane), warps 2..9 = epilogue (TMEM -> registers -> +bias -> HBM).  Two accumulator stages
 // in TMEM let the epilogue of tile t overlap the MMAs of tile t+1; a ring of smem stages
-// decouples TMA from the MMAs.  Persistent: grid = min(#SM, tiles), tiles strided over the CTAs.
+// decouples TMA from the MMAs.  Persistent: at most one CTA pair per two SMs, tiles strided over the pairs.
 #pragma once
 
 #include <cuda.h>
@@ -26,21 +26,6 @@ constexpr int BLOCK_K = 32;    // tf32 elements per 128-byte swizzle row
 constexpr int UMMA_K = 8;      // tf32 elements one tcgen05.mma consumes along K (32 bytes)
 constexpr int EPI_WARPS = 8;    // two warps per TMEM lane quarter, each draining every other 32-row chunk
 constexpr int NTHREADS = 64 + 32 * EPI_WARPS;
-
-template <int NB>
-struct ScoreCfg {
-  static_assert(NB == 64 || NB == 128 || NB == 256, "batch chunk must be 64, 128 or 256 rows");
-  static constexpr int A_BYTES = TILE_M * BLOCK_K * 4;
-  static constexpr int B_BYTES = NB * BLOCK_K * 4;
-  static constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  static constexpr int STAGES = (200 * 1024 / STAGE_BYTES) > 8 ? 8 : (200 * 1024 / STAGE_BYTES);
-  static constexpr int BAR_BYTES = 256;
-  static constexpr int SMEM = STAGES * STAGE_BYTES + BAR_BYTES + 1024;   // + slack to align to 1024
-  static constexpr int TMEM_COLS = 2 * NB;                               // two accumulator stages
-  // instruction descriptor (kind::tf32): D = f32, A = B = tf32, both K-major, N = NB, M = 128
-  static constexpr uint32_t IDESC = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(NB >> 3) << 17) |
-                                    ((uint32_t)(TILE_M >> 4) << 24);
-};
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -168,115 +153,11 @@ struct ScoreArgs {
   int n_chunks;          // ceil(B / NB)
 };
 
-template <int NB>
-__global__ void __launch_bounds__(NTHREADS, 1)
-k_score_tc(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_h, ScoreArgs a) {
-  using C = ScoreCfg<NB>;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + C::STAGES * C::STAGE_BYTES);
-  uint64_t* full = bars;                      // [STAGES] TMA -> MMA
-  uint64_t* empty = bars + C::STAGES;         // [STAGES] MMA -> TMA
-  uint64_t* tfull = bars + 2 * C::STAGES;     // [2] MMA -> epilogue
-  uint64_t* tempty = tfull + 2;               // [2] epilogue -> MMA
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(tempty + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int total = a.n_mtiles * a.n_chunks;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < C::STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(&tfull[s], 1); mbar_init(&tempty[s], EPI_WARPS); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_holder)), "r"((uint32_t)C::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *reinterpret_cast<volatile uint32_t*>(tmem_holder);
-
-  if (warp == 0) {
-    int stage = 0; uint32_t phase = 0;
-    for (int t = blockIdx.x; t < total; t += gridDim.x) {
-      const int m = t / a.n_chunks, n = t - m * a.n_chunks;
-      for (int k = 0; k < a.num_k; ++k) {
-        mbar_wait(&empty[stage], phase ^ 1u);
-        if (elect_one()) {
-          uint8_t* sa = smem + stage * C::STAGE_BYTES;
-          mbar_expect_tx(&full[stage], (uint32_t)C::STAGE_BYTES);
-          tma_load_2d(sa, &map_w, &full[stage], k * BLOCK_K, m * TILE_M);
-          tma_load_2d(sa + C::A_BYTES, &map_h, &full[stage], k * BLOCK_K, n * NB);
-        }
-        __syncwarp();
-        if (++stage == C::STAGES) { stage = 0; phase ^= 1u; }
-      }
-    }
-  } else if (warp == 1) {
-    int stage = 0; uint32_t phase = 0;
-    int acc = 0; uint32_t acc_phase = 0;
-    for (int t = blockIdx.x; t < total; t += gridDim.x) {
-      mbar_wait(&tempty[acc], acc_phase ^ 1u);
-      tcgen05_fence_after();
-      const uint32_t d_tmem = tmem_base + (uint32_t)(acc * NB);
-      for (int k = 0; k < a.num_k; ++k) {
-        mbar_wait(&full[stage], phase);
-        tcgen05_fence_after();
-        if (elect_one()) {
-          const uint8_t* sa = smem + stage * C::STAGE_BYTES;
-          const uint64_t da = make_desc(sa), db = make_desc(sa + C::A_BYTES);
-#pragma unroll
-          for (int kk = 0; kk < BLOCK_K / UMMA_K; ++kk)   // +32 bytes along K inside the swizzle row
-            umma_tf32(d_tmem, da + (uint64_t)(kk * 2), db + (uint64_t)(kk * 2), C::IDESC, (uint32_t)((k | kk) != 0));
-          umma_commit(&empty[stage]);
-          if (k == a.num_k - 1) umma_commit(&tfull[acc]);
-        }
-        __syncwarp();
-        if (++stage == C::STAGES) { stage = 0; phase ^= 1u; }
-      }
-      acc ^= 1; if (acc == 0) acc_phase ^= 1u;
-    }
-  } else {
-    const int q = warp & 3;                   // the TMEM lane quarter this warp may read
-    int acc = 0; uint32_t acc_phase = 0;
-    for (int t = blockIdx.x; t < total; t += gridDim.x) {
-      const int m = t / a.n_chunks, n = t - m * a.n_chunks;
-      mbar_wait(&tfull[acc], acc_phase);
-      tcgen05_fence_after();
-      const int c = m * TILE_M + q * 32 + lane;
-      const bool cok = c < a.n_cols;
-      const float bv = cok ? __ldg(a.bias + c) : 0.f;
-      const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * NB);
-#pragma unroll 1
-      for (int j = (warp - 2) >> 2; j < NB / 32; j += EPI_WARPS / 4) {
-        const int row0 = n * NB + j * 32;
-        if (row0 >= a.n_rows) break;          // warp-uniform
-        uint32_t r[32];
-        tmem_ld32(tbase + (uint32_t)(j * 32), r);
-        tmem_wait_ld();
-        store_rows(a.out + (long long)row0 * a.ldo + c, a.ldo, r, bv, cok, min(32, a.n_rows - row0));
-      }
-      tcgen05_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&tempty[acc]);
-      acc ^= 1; if (acc == 0) acc_phase ^= 1u;
-    }
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"((uint32_t)C::TMEM_COLS) : "memory");
-  }
-}
-
 // ============================================================================================
-// The same GEMM on CTA pairs (tcgen05 cta_group::2, thread-block cluster of 2): the two SMs of a
+// CTA pairs (tcgen05 cta_group::2, thread-block cluster of 2): the two SMs of a
 // pair compute one 256-column x NB-row tile. Each CTA loads its own 128 catalogue columns of A
 // and HALF of the batch-row operand B; the pair's tensor cores read both halves, so the operand
-// bytes per MMA drop from 48 KB to 32 KB per SM and k-block - the single-CTA kernel is bound by
+// bytes per MMA drop from 48 KB to 32 KB per SM and k-block - one CTA per tile is bound by
 // exactly that feed (profiles/r01_ncu_full_k_score_tc_v1.txt). Protocol:
 //   * TMA of both CTAs completes on the LEADER's (cluster rank 0) full barrier;
 //   * the leader's elected thread issues the MMAs for the pair and commits with a multicast
@@ -467,33 +348,18 @@ inline EncodeTiledFn encode_fn() {
 }
 
 // K-major fp32 matrix [rows, hp] (row stride hp floats) cut into [box_rows x 32] boxes, 128-byte swizzle.
-// as_tf32: the copy engine rounds fp32 to tf32 on the way in (the MMA alone would truncate).
-inline int make_map(CUtensorMap* map, const float* base, int hp, long long rows, int box_rows, bool as_tf32) {
+// The copy engine rounds fp32 to tf32 on the way in (the MMA alone would truncate).
+inline int make_map(CUtensorMap* map, const float* base, int hp, long long rows, int box_rows) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) return fail(OCF_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
   cuuint64_t gdim[2] = {(cuuint64_t)hp, (cuuint64_t)rows};
   cuuint64_t gstride[1] = {(cuuint64_t)hp * sizeof(float)};
   cuuint32_t box[2] = {(cuuint32_t)BLOCK_K, (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(map, as_tf32 ? CU_TENSOR_MAP_DATA_TYPE_TFLOAT32 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+  CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_TFLOAT32, 2,
                   const_cast<float*>(base), gdim, gstride, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(OCF_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult " + std::to_string((int)r));
-  return OCF_OK;
-}
-
-template <int NB>
-inline int launch_score_nb(const CUtensorMap& mw, const CUtensorMap& mh, const ScoreArgs& a, int sm_count, cudaStream_t st) {
-  using C = ScoreCfg<NB>;
-  static bool attr_set = false;
-  if (!attr_set) {
-    OCF_CUDA(cudaFuncSetAttribute(k_score_tc<NB>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM));
-    attr_set = true;
-  }
-  const int total = a.n_mtiles * a.n_chunks;
-  const int grid = total < sm_count ? total : sm_count;
-  k_score_tc<NB><<<grid, NTHREADS, C::SMEM, st>>>(mw, mh, a);
-  OCF_LAUNCHED();
   return OCF_OK;
 }
 

@@ -1,4 +1,4 @@
-"""Summary of the bench lines a scripts/gpu_quick.sh (or gpu_r02c.sh) call left in gpurun_out/: python scripts/show_quick.py TAG [SUFFIX...]"""
+"""Summary of the bench lines a scripts/gpu_quick.sh call left behind: python scripts/show_quick.py TAG [SUFFIX...]"""
 import json, sys
 tag = sys.argv[1]
 sfxs = sys.argv[2:] or [""]
