@@ -1011,12 +1011,14 @@ __global__ void __launch_bounds__(256) k_sort_alloc(SortArgs a) {
   if (c < a.n_cols) {
     n = a.cnt[c];
     if (n > 0) {
-      const int any = a.dense ? 0xff : a.codeor[c];      // dense updates touch every array of every column
+      // dense updates touch every array of every column, including an input block no rating feeds (the "zeros" aux
+      // block, bit 0): k_row_update's dense walk leaves all arrays of a heavy column to the heavy list
+      const int any = a.dense ? 0xff : a.codeor[c];
       if (a.do_dec && (any & CODE_TGT)) arr[n_arr++] = 0;
       if (a.do_enc)
         for (int blk = 0; blk < a.nblk; ++blk) {
           const int bit = blk == 0 ? a.bits3.x : (blk == 1 ? a.bits3.y : a.bits3.z);
-          if (any & bit) arr[n_arr++] = 1 + blk;
+          if (a.dense || (any & bit)) arr[n_arr++] = 1 + blk;
         }
       if (!a.dense) n_tasks = n_arr;
     }
