@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define OCF_VERSION 100
+#define OCF_VERSION 101
 
 typedef enum {
   OCF_OK = 0,
@@ -46,7 +46,7 @@ typedef enum { OCF_LOSS_MSE = 0, OCF_LOSS_MAE = 1 } ocf_loss;
 /* optimizer, train.py:50-51 / train_jester.py:61 */
 typedef enum { OCF_OPT_SGD = 0, OCF_OPT_ADAGRAD, OCF_OPT_RMSPROP, OCF_OPT_ADAM } ocf_optimizer;
 
-typedef struct ocf_store ocf_store;   /* device-resident rating store (CSR + CSC)            */
+typedef struct ocf_store ocf_store;   /* device-resident rating store (CSR)                  */
 typedef struct ocf_pair ocf_pair;     /* (input store, target store) of a fixed-split set    */
 typedef struct ocf_batch ocf_batch;   /* one batch: row ids, keep-flags, gathered tiles      */
 typedef struct ocf_model ocf_model;   /* weights, optimizer state, workspaces                */
@@ -68,15 +68,13 @@ int ocf_host_free(void* ptr);
  * by the caller: `col` already holds dense columns). Rows keep their stored order: draw j of
  * the reciprocal dropout belongs to the j-th stored rating (data_reader.py:130-134).
  * Repeated columns inside a row are allowed and resolve last-write-wins like the dense fills
- * at data_reader.py:158-169. `build_csc` != 0 marks a store that will be trained on: if some row
- * repeats a column, the column-major index the training update then needs is built too.
+ * at data_reader.py:158-169.
  * Limits: nnz < 2^31, n_cols < 2^31. */
 int ocf_store_create(int64_t n_rows, int64_t n_cols, const int64_t* rowptr, const int32_t* col,
-                     const float* val, int build_csc, ocf_store** out);
+                     const float* val, ocf_store** out);
 int ocf_store_destroy(ocf_store* store);
-/* info[0]=n_rows, [1]=n_cols, [2]=nnz, [3]=1 if any row repeats a column, [4]=longest column,
- * [5]=device bytes held */
-int ocf_store_info(const ocf_store* store, int64_t info[6]);
+/* info[0]=n_rows, [1]=n_cols, [2]=nnz, [3]=1 if any row repeats a column, [4]=device bytes held */
+int ocf_store_info(const ocf_store* store, int64_t info[5]);
 
 /* Fixed-split valid/test set: row r of `in_store` holds the inputs of row r of `tgt_store`
  * (user_dicts_valid[0]/[1], data_reader.py:372-380; a None input row is an empty row). */

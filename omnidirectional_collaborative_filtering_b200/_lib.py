@@ -55,7 +55,7 @@ _SIGNATURES = {
     "ocf_kernel_launches": (C.c_int64, []),
     "ocf_host_alloc": (C.c_int, [C.c_int64, C.POINTER(_P)]),
     "ocf_host_free": (C.c_int, [_P]),
-    "ocf_store_create": (C.c_int, [C.c_int64, C.c_int64, _P, _P, _P, C.c_int, C.POINTER(_P)]),
+    "ocf_store_create": (C.c_int, [C.c_int64, C.c_int64, _P, _P, _P, C.POINTER(_P)]),
     "ocf_store_destroy": (C.c_int, [_P]),
     "ocf_store_info": (C.c_int, [_P, C.POINTER(C.c_int64)]),
     "ocf_pair_create": (C.c_int, [_P, _P, C.POINTER(_P)]),

@@ -108,8 +108,8 @@ struct ocf_comm {
 // handles
 // ============================================================================================
 struct ocf_store {
-  int64_t n_rows = 0, n_cols = 0, nnz = 0, max_col_len = 0;
-  bool has_dups = false, has_csc = false;
+  int64_t n_rows = 0, n_cols = 0, nnz = 0;
+  bool has_dups = false;
   std::vector<int64_t> h_rowptr;
   StoreDev dev{};
   Arena mem;
@@ -156,7 +156,7 @@ struct ocf_pair {
 // a batch object owns another when its column grouping runs AHEAD of the step on the batch's own stream.
 struct WorkList {
   uint32_t* matches = nullptr;    // [3 * entries] (batch row | code << 16, value, entry)
-  int32_t* mcol = nullptr;        // [entries] CSC scan only
+  int64_t entries = 0;            //   capacity of `matches` in records
   int2* seg = nullptr;            // [n_cols] dense mode: (first match, matches) of every column
   int4* tasks = nullptr;          // [(nblk + 1) * n_cols]
   int4* heavy = nullptr;          //   tasks with more than HEAVY_N matches
@@ -168,10 +168,10 @@ struct WorkList {
 
 // What a work list depends on besides the batch's own tiles.
 struct WorkSig {
-  int n_cols = 0, nblk = 0, b0 = 0, b1 = 0, b2 = 0, do_dec = 0, do_enc = 0, dense = 0, heavy = 0, B = 0;
+  int n_cols = 0, nblk = 0, b0 = 0, b1 = 0, b2 = 0, do_dec = 0, do_enc = 0, dense = 0, heavy = 0, B = 0, dups = 0;
   bool operator==(const WorkSig& o) const {
     return n_cols == o.n_cols && nblk == o.nblk && b0 == o.b0 && b1 == o.b1 && b2 == o.b2 && do_dec == o.do_dec &&
-           do_enc == o.do_enc && dense == o.dense && heavy == o.heavy && B == o.B;
+           do_enc == o.do_enc && dense == o.dense && heavy == o.heavy && B == o.B && dups == o.dups;
   }
 };
 
@@ -195,9 +195,6 @@ struct ocf_batch {
   int32_t* d_ent_col = nullptr;
   float* d_ent_val = nullptr;
   uint8_t* d_codes = nullptr;
-  uint32_t* d_rowslot = nullptr;
-  int64_t rowslot_rows = 0;
-  uint32_t tag = 0;
   BatchDev dev{};
   int mode = 0;                   // 0 empty, 1 split, 2 fixed
   const ocf_store* store = nullptr;
@@ -259,20 +256,19 @@ struct ocf_model {
   StepDev step_mirror{};          //   what the device holds once everything enqueued so far has run
   bool step_mirror_valid = false;
   TailBuf tail{};                 // row-tail counters and group sums of K2 / K3
-  // captured steps (CUDA graphs), keyed by batch object / rows / kind; dropped whenever anything they
+  // captured steps (CUDA graphs), keyed by batch object / rows / kind / whether the batch's store repeats a
+  // column (K4a clears the match list first then); dropped whenever anything they
   // bake in changes (workspaces, optimizer, trainable flags, ...)
   struct StepGraph { cudaGraphExec_t exec = nullptr; int kernels = 0; int seen = 0; bool failed = false; };
-  std::map<std::tuple<uint64_t, int, int, int, int>, StepGraph> graphs;
+  std::map<std::tuple<uint64_t, int, int, int, int, int>, StepGraph> graphs;
   cudaStream_t cap = nullptr;     // capture stream
   bool capturing = false;
-  int* d_err = nullptr;
   int64_t steps_logged = 0;
   cudaEvent_t step_ev[64] = {nullptr};
   uint32_t* col_matches = nullptr;
-  int32_t* col_mcol = nullptr;
   int2* col_seg = nullptr;
   int4* col_tasks = nullptr;
-  int4* col_heavy = nullptr;      // tasks with more than HEAVY_N matches (batch-side K4a only), same capacity as col_tasks
+  int4* col_heavy = nullptr;      // tasks with more than HEAVY_N matches, same capacity as col_tasks
   int* col_counters = nullptr;
   int32_t* topk_cols = nullptr;   // top-k epilogue outputs [max_rows, 512] (allocated with dense_out's arena)
   float* topk_scores = nullptr;
@@ -412,7 +408,7 @@ extern "C" int ocf_profile_read(int tag, double* total_ms, int64_t* count) {
 // store
 // ============================================================================================
 extern "C" int ocf_store_create(int64_t n_rows, int64_t n_cols, const int64_t* rowptr, const int32_t* col,
-                                const float* val, int build_csc, ocf_store** out) {
+                                const float* val, ocf_store** out) {
   OCF_REQUIRE(out != nullptr && rowptr != nullptr, "ocf_store_create: null argument");
   *out = nullptr;
   OCF_REQUIRE(n_rows >= 0 && n_cols > 0 && n_cols < (int64_t(1) << 31), "ocf_store_create: bad shape");
@@ -467,68 +463,6 @@ extern "C" int ocf_store_create(int64_t n_rows, int64_t n_cols, const int64_t* r
       return bail(fail(OCF_ERR_CUDA, "ocf_store_create: upload failed"));
   }
   s->dev.rowptr = d_rowptr; s->dev.col = d_col; s->dev.val = d_val; s->dev.next_dup = d_nd;
-  if (build_csc && s->has_dups) {
-    // (only stores whose rows repeat a column train through the CSC scan; all others build their
-    // update work list from the batch alone and never need the column-major index)
-    // counting sort in CSR order: entries of a column come out ordered by (row, position)
-    std::vector<int64_t> colptr((size_t)n_cols + 1, 0);
-    for (int64_t e = 0; e < nnz; ++e) colptr[(size_t)col[e] + 1]++;
-    for (int64_t c = 0; c < n_cols; ++c) {
-      s->max_col_len = std::max(s->max_col_len, colptr[c + 1]);
-      colptr[c + 1] += colptr[c];
-    }
-    std::vector<int64_t> cursor(colptr.begin(), colptr.end() - 1);
-    std::vector<int32_t> crow((size_t)nnz), cj((size_t)nnz);
-    for (int64_t r = 0; r < n_rows; ++r)
-      for (int64_t e = rowptr[r]; e < rowptr[r + 1]; ++e) {
-        const int64_t k = cursor[col[e]]++;
-        crow[k] = (int32_t)r;
-        cj[k] = (int32_t)(e - rowptr[r]);
-      }
-    int64_t* d_colptr = nullptr; int32_t* d_crow = nullptr; int32_t* d_cj = nullptr;
-    if ((st = s->mem.get(&d_colptr, (size_t)n_cols + 1)) || (st = s->mem.get(&d_crow, (size_t)nnz)) ||
-        (st = s->mem.get(&d_cj, (size_t)nnz)))
-      return bail(st);
-    if (cudaMemcpy(d_colptr, colptr.data(), sizeof(int64_t) * (n_cols + 1), cudaMemcpyHostToDevice) != cudaSuccess ||
-        (nnz && cudaMemcpy(d_crow, crow.data(), sizeof(int32_t) * nnz, cudaMemcpyHostToDevice) != cudaSuccess) ||
-        (nnz && cudaMemcpy(d_cj, cj.data(), sizeof(int32_t) * nnz, cudaMemcpyHostToDevice) != cudaSuccess))
-      return bail(fail(OCF_ERR_CUDA, "ocf_store_create: upload failed"));
-    s->dev.colptr = d_colptr; s->dev.crow = d_crow; s->dev.cj = d_cj;
-    // scan schedule: consecutive columns grouped up to SCAN_T entries (a longer column is its own
-    // group); groups with the most entries first so the long ones start early
-    std::vector<int2> groups;
-    int scan_t = SCAN_SUB;
-    while (scan_t < SCAN_T_MAX && nnz / scan_t > 148 * 5 * 3 / 2) scan_t *= 2;   // about one group per resident CTA
-    {
-      const int64_t SCAN_T = scan_t;
-      int64_t c0 = 0;
-      while (c0 < n_cols) {
-        int64_t c1 = c0 + 1;
-        while (c1 < n_cols && colptr[c1 + 1] - colptr[c0] <= SCAN_T) ++c1;
-        if (colptr[c1] > colptr[c0]) groups.push_back(make_int2((int)c0, (int)c1));
-        c0 = c1;
-      }
-      std::stable_sort(groups.begin(), groups.end(), [&](const int2& x, const int2& y) {
-        return colptr[x.y] - colptr[x.x] > colptr[y.y] - colptr[y.x];
-      });
-    }
-    int2* d_groups = nullptr;
-    if ((st = s->mem.get(&d_groups, groups.size()))) return bail(st);
-    if (!groups.empty() && cudaMemcpy(d_groups, groups.data(), sizeof(int2) * groups.size(), cudaMemcpyHostToDevice) != cudaSuccess)
-      return bail(fail(OCF_ERR_CUDA, "ocf_store_create: upload failed"));
-    s->dev.groups = d_groups;
-    s->dev.n_groups = (int)groups.size();
-    s->dev.scan_t = scan_t;
-    std::vector<int32_t> ccol((size_t)nnz);
-    for (int64_t c = 0; c < n_cols; ++c)
-      for (int64_t e = colptr[c]; e < colptr[c + 1]; ++e) ccol[e] = (int32_t)c;
-    int32_t* d_ccol = nullptr;
-    if ((st = s->mem.get(&d_ccol, (size_t)nnz))) return bail(st);
-    if (nnz && cudaMemcpy(d_ccol, ccol.data(), sizeof(int32_t) * nnz, cudaMemcpyHostToDevice) != cudaSuccess)
-      return bail(fail(OCF_ERR_CUDA, "ocf_store_create: upload failed"));
-    s->dev.ccol = d_ccol;
-    s->has_csc = true;
-  }
   *out = s;
   return OCF_OK;
 }
@@ -538,10 +472,10 @@ extern "C" int ocf_store_destroy(ocf_store* s) {
   return OCF_OK;
 }
 
-extern "C" int ocf_store_info(const ocf_store* s, int64_t info[6]) {
+extern "C" int ocf_store_info(const ocf_store* s, int64_t info[5]) {
   OCF_REQUIRE(s && info, "ocf_store_info: null argument");
   info[0] = s->n_rows; info[1] = s->n_cols; info[2] = s->nnz; info[3] = s->has_dups ? 1 : 0;
-  info[4] = s->max_col_len; info[5] = (int64_t)s->mem.bytes;
+  info[4] = (int64_t)s->mem.bytes;
   return OCF_OK;
 }
 
@@ -663,7 +597,6 @@ extern "C" int ocf_batch_destroy(ocf_batch* b) {
     if (b->wl_graph) cudaGraphExecDestroy(b->wl_graph);
     b->wl_mem.release();
     b->mem.release();
-    if (b->d_rowslot) cudaFree(b->d_rowslot);
     if (b->h_staging) cudaFreeHost(b->h_staging);
     if (b->copied) cudaEventDestroy(b->copied);
     delete b;
@@ -684,7 +617,7 @@ static int pick_chunk(int64_t n_entries) {
 // leaves the flags to the device.
 static int batch_stage(ocf_batch* b, const int32_t* row_ids, int n_rows, const std::vector<int64_t>& rp_a,
                        const std::vector<int64_t>* rp_b, int64_t n_store_rows, const uint8_t* flags,
-                       int64_t n_flags, cudaStream_t stream, uint32_t hdr_tag, int hdr_pass_through, float hdr_aux,
+                       int64_t n_flags, cudaStream_t stream, int hdr_pass_through, float hdr_aux,
                        bool with_draws = false, const int64_t* draw_len = nullptr) {
   OCF_REQUIRE(n_rows > 0 && n_rows <= b->max_rows, "batch fill: row count exceeds the batch capacity");
   if (b->copy_pending) { OCF_CUDA(cudaEventSynchronize(b->copied)); b->copy_pending = false; }
@@ -732,7 +665,7 @@ static int batch_stage(ocf_batch* b, const int32_t* row_ids, int n_rows, const s
   }
   h_eoff[n_rows] = (int32_t)e; h_iptr[n_rows] = it;
   h_hdr->B = n_rows; h_hdr->n_items = (int)n_items; h_hdr->n_entries = (int)total;
-  h_hdr->tag = hdr_tag; h_hdr->cdf_row0 = b->cdf0_row0; h_hdr->pass_through = hdr_pass_through;
+  h_hdr->cdf_row0 = b->cdf0_row0; h_hdr->pass_through = hdr_pass_through;
   h_hdr->rng_lo = b->rng_lo; h_hdr->rng_range = b->rng_range; h_hdr->aux_value = hdr_aux;
   h_hdr->word_base = b->word_base; h_hdr->ring_words = b->ring_words;
   if (flags != nullptr && total > 0) std::memcpy(hs + off[7], flags, (size_t)total);
@@ -782,7 +715,13 @@ static int batch_release(const ocf_batch* cb, cudaStream_t st) {
   return OCF_OK;
 }
 
-static int prepare_rowslot(ocf_batch* b, const ocf_store* store, const int32_t* row_ids, int32_t n_rows, cudaStream_t stream, const char* who);
+// Caller input check of the split fills: a batch lists every row at most once.
+static int check_distinct_rows(const int32_t* row_ids, int32_t n_rows, const char* who) {
+  std::vector<int32_t> tmp(row_ids, row_ids + std::max(n_rows, 0));
+  std::sort(tmp.begin(), tmp.end());
+  if (std::adjacent_find(tmp.begin(), tmp.end()) != tmp.end()) return fail(OCF_ERR_INVALID, std::string(who) + ": a row appears twice in the batch");
+  return OCF_OK;
+}
 
 extern "C" int ocf_batch_fill_split(ocf_batch* b, const ocf_store* store, const int32_t* row_ids, int32_t n_rows,
                                     const uint8_t* keep_flags, int64_t n_flags, int pass_through,
@@ -791,11 +730,9 @@ extern "C" int ocf_batch_fill_split(ocf_batch* b, const ocf_store* store, const 
   OCF_REQUIRE(keep_flags != nullptr || n_flags == 0, "ocf_batch_fill_split: null keep_flags");
   cudaStream_t user = as_stream(stream_);
   cudaStream_t stream = fill_begin(b);
-  OCF_TRY(prepare_rowslot(b, store, row_ids, n_rows, stream, "ocf_batch_fill_split"));
+  OCF_TRY(check_distinct_rows(row_ids, n_rows, "ocf_batch_fill_split"));
   OCF_TRY(batch_stage(b, row_ids, n_rows, store->h_rowptr, nullptr, store->n_rows, keep_flags, n_flags, stream,
-                      b->tag, pass_through ? 1 : 0, aux_var_value));
-  b->dev.rowslot = b->d_rowslot;
-  b->dev.tag = b->tag;
+                      pass_through ? 1 : 0, aux_var_value));
   b->mode = 1; b->store = store; b->aux_value = aux_var_value; b->rng_mode = false;
   // in split mode every listed rating is a target when pass_through, else the flag-0 ones
   int64_t tc = 0;
@@ -842,8 +779,7 @@ extern "C" int ocf_batch_fill_fixed(ocf_batch* b, const ocf_pair* pair, const in
   cudaStream_t user = as_stream(stream_);
   cudaStream_t stream = fill_begin(b);
   OCF_TRY(batch_stage(b, row_ids, n_rows, pair->in->h_rowptr, &pair->tg->h_rowptr, pair->in->n_rows, nullptr, -1, stream,
-                      0u, 0, aux_var_value));
-  b->dev.rowslot = nullptr; b->dev.tag = 0;
+                      0, aux_var_value));
   b->mode = 2; b->store = pair->tg; b->aux_value = aux_var_value;
   b->pair = pair;
   OCF_TRY(launch_gather(b, stream));
@@ -1085,26 +1021,6 @@ extern "C" int ocf_store_set_orig_pos(ocf_store* s, const int32_t* orig_pos) {
   return OCF_OK;
 }
 
-static int prepare_rowslot(ocf_batch* b, const ocf_store* store, const int32_t* row_ids, int32_t n_rows, cudaStream_t stream, const char* who) {
-  {  // the row -> slot map needs distinct rows
-    std::vector<int32_t> tmp(row_ids, row_ids + std::max(n_rows, 0));
-    std::sort(tmp.begin(), tmp.end());
-    if (std::adjacent_find(tmp.begin(), tmp.end()) != tmp.end()) return fail(OCF_ERR_INVALID, std::string(who) + ": a row appears twice in the batch");
-  }
-  if (b->rowslot_rows < store->n_rows) {
-    if (b->d_rowslot) { OCF_CUDA(cudaStreamSynchronize(stream)); cudaFree(b->d_rowslot); b->d_rowslot = nullptr; }
-    OCF_CUDA(cudaMalloc(reinterpret_cast<void**>(&b->d_rowslot), sizeof(uint32_t) * (size_t)std::max<int64_t>(store->n_rows, 1)));
-    b->rowslot_rows = store->n_rows;
-    b->tag = 0;
-  }
-  if (b->tag == 0 || b->tag >= (1u << (32 - SLOT_BITS)) - 1 || b->store != store) {
-    OCF_CUDA(cudaMemsetAsync(b->d_rowslot, 0, sizeof(uint32_t) * (size_t)std::max<int64_t>(b->rowslot_rows, 1), stream));
-    b->tag = 0;
-  }
-  b->tag += 1;
-  return OCF_OK;
-}
-
 extern "C" int ocf_batch_fill_split_rng(ocf_batch* b, const ocf_store* store, const int32_t* row_ids, int32_t n_rows,
                                         ocf_rng* rng, double lo, double hi, const int64_t* full_len, int pass_through,
                                         float aux_var_value, const ocf_rng_slice* slice, void* stream_) {
@@ -1141,11 +1057,9 @@ extern "C" int ocf_batch_fill_split_rng(ocf_batch* b, const ocf_store* store, co
   OCF_TRY(rng_enqueue_blocks(rng, kb1));
   if (rng->next_block <= kb1) return fail(OCF_ERR_STATE, "ocf_batch_fill_split_rng: the stream ring is too small for this batch");
   b->d_words = rng->d_ring; b->word_base = (uint32_t)(u0 % rng->RW); b->ring_words = (uint32_t)rng->RW;
-  OCF_TRY(prepare_rowslot(b, store, row_ids, n_rows, stream, "ocf_batch_fill_split_rng"));
+  OCF_TRY(check_distinct_rows(row_ids, n_rows, "ocf_batch_fill_split_rng"));
   OCF_TRY(batch_stage(b, row_ids, n_rows, store->h_rowptr, nullptr, store->n_rows, nullptr, -1, stream,
-                      b->tag, pass_through ? 1 : 0, aux_var_value, true, full_len));
-  b->dev.rowslot = b->d_rowslot;
-  b->dev.tag = b->tag;
+                      pass_through ? 1 : 0, aux_var_value, true, full_len));
   b->mode = 1; b->store = store; b->aux_value = aux_var_value; b->rng_mode = true;
   b->pass_through = pass_through ? 1 : 0;
   b->target_count = pass_through ? b->dev.n_entries : -1;      // the flags never visit the host
@@ -1262,7 +1176,6 @@ static int alloc_workspace(ocf_model* m, int max_rows, int64_t max_entries) {
   OCF_TRY(ws.get(&m->rowstats, (size_t)max_rows * ROWSTAT_W + (size_t)max_rows * m->hp[L - 1], true));
   m->dh_top = m->rowstats + (size_t)max_rows * ROWSTAT_W;
   OCF_TRY(ws.get(&m->col_matches, (size_t)max_entries * 3));
-  OCF_TRY(ws.get(&m->col_mcol, (size_t)max_entries));
   m->col_bits_words = (size_t)m->cfg.n_cols * (size_t)((max_rows + 31) / 32);
   OCF_TRY(ws.get(&m->col_bits, m->col_bits_words, true));
   return OCF_OK;
@@ -1301,7 +1214,7 @@ extern "C" int ocf_model_create(const ocf_model_config* cfg, ocf_model** out) {
   }
   if (st) return bail(st);
   if ((st = m->mem.get(&m->regparts, (size_t)N_REGPART * (L + 1), true)) || (st = m->mem.get(&m->d_step, 1, true)) ||
-      (st = m->mem.get(&m->d_err, 1, true)) || (st = m->mem.get(&m->col_tasks, (size_t)N * (m->nblk + 1))) || (st = m->mem.get(&m->col_heavy, (size_t)N * (m->nblk + 1))) || (st = m->mem.get(&m->col_seg, (size_t)N, true)) ||
+      (st = m->mem.get(&m->col_tasks, (size_t)N * (m->nblk + 1))) || (st = m->mem.get(&m->col_heavy, (size_t)N * (m->nblk + 1))) || (st = m->mem.get(&m->col_seg, (size_t)N, true)) ||
       (st = m->mem.get(&m->col_counters, 8, true)) || (st = m->mem.get(&m->col_state, (size_t)2 * N, true)) ||
       (st = m->mem.get(&m->col_info, (size_t)N)))
     return bail(st);
@@ -1548,8 +1461,6 @@ static int check_step(const ocf_model* m, const ocf_batch* b, bool train) {
   OCF_REQUIRE(m && b, "step: null argument");
   if (b->mode == 0) return fail(OCF_ERR_STATE, "step: the batch has not been filled");
   if (train && b->mode != 1) return fail(OCF_ERR_STATE, "train step needs a split batch (ocf_batch_fill_split)");
-  if (train && b->store->has_dups && !b->store->has_csc)
-    return fail(OCF_ERR_STATE, "training on a store whose rows repeat a column needs the store's column index (build_csc)");
   OCF_REQUIRE(b->store->n_cols == m->cfg.n_cols, "step: the batch's store and the model disagree on n_cols");
   OCF_REQUIRE(b->dev.B <= m->cfg.max_rows && b->dev.n_entries <= m->cfg.max_entries && b->dev.n_items <= m->max_items,
               "step: the batch exceeds the model's workspace");
@@ -1784,7 +1695,7 @@ static bool heavy_model(const ocf_model* m) {
 // The model's own work list (filled inside the step).
 static WorkList model_wl(const ocf_model* m) {
   WorkList w;
-  w.matches = m->col_matches; w.mcol = m->col_mcol; w.seg = m->col_seg; w.tasks = m->col_tasks; w.heavy = m->col_heavy;
+  w.matches = m->col_matches; w.entries = m->cfg.max_entries; w.seg = m->col_seg; w.tasks = m->col_tasks; w.heavy = m->col_heavy;
   w.counters = m->col_counters; w.state = m->col_state; w.info = m->col_info; w.bits = m->col_bits;
   return w;
 }
@@ -1793,7 +1704,7 @@ static WorkSig work_sig(const ocf_model* m, const ocf_batch* b) {
   WorkSig s;
   s.n_cols = m->cfg.n_cols; s.nblk = m->nblk; s.b0 = m->bits.x; s.b1 = m->bits.y; s.b2 = m->bits.z;
   s.do_dec = m->layers[m->L].trainable ? 1 : 0; s.do_enc = m->layers[0].trainable ? 1 : 0;
-  s.dense = make_opt(m).dense; s.heavy = heavy_model(m) ? 1 : 0; s.B = b->dev.B;
+  s.dense = make_opt(m).dense; s.heavy = heavy_model(m) ? 1 : 0; s.B = b->dev.B; s.dups = b->store->has_dups ? 1 : 0;
   return s;
 }
 // The batch carries the work list of its current fill, built for this model's settings.
@@ -1813,47 +1724,30 @@ static int launch_scan(ocf_model* m, const ocf_batch* b, int do_dec, int do_enc,
     OCF_CUDA(cudaMemsetAsync(wl.counters, 0, 8 * sizeof(int), st));
     if (dense) OCF_CUDA(cudaMemsetAsync(wl.seg, 0, sizeof(int2) * (size_t)m->cfg.n_cols, st));
   }
-  if (!b->store->has_dups) {
-    // batch-side counting sort (every (column, batch row) pair is unique)
-    const int W = (bt.B + 31) / 32;
-    const size_t N = (size_t)m->cfg.n_cols;
-    if (!zeroed) {
-      OCF_CUDA(cudaMemsetAsync(wl.state, 0, sizeof(int) * 2 * N, st));
-      OCF_CUDA(cudaMemsetAsync(wl.bits, 0, sizeof(uint32_t) * N * W, st));
-    }
-    SortArgs a{};
-    a.bt = bt;
-    a.cnt = wl.state; a.codeor = wl.state + N;
-    a.colinfo = wl.info; a.bits = wl.bits; a.W = W; a.counters = wl.counters;
-    a.matches = wl.matches; a.tasks = wl.tasks; a.colseg = wl.seg; a.heavy = heavy_model(m) ? wl.heavy : nullptr;
-    a.n_cols = m->cfg.n_cols; a.nblk = m->nblk; a.bits3 = m->bits; a.dense = dense; a.do_dec = do_dec; a.do_enc = do_enc;
-    const int grid = item_grid(m, b);
-    g_prof.begin(3, st);
-    k_sort_count<<<grid, 128, 0, st>>>(a);
-    OCF_LAUNCHED();
-    OCF_CUDA(launch_pdl(!g_prof.on, k_sort_alloc, dim3((m->cfg.n_cols + 255) / 256), dim3(256), st, a));
-    OCF_LAUNCHED();
-    OCF_CUDA(launch_pdl(!g_prof.on, k_sort_place, dim3(grid), dim3(128), st, a));
-    OCF_LAUNCHED();
-    g_prof.end(3, st);
-    return OCF_OK;
+  const int dups = b->store->has_dups ? 1 : 0;
+  const int W = (bt.B + 31) / 32;
+  const size_t N = (size_t)m->cfg.n_cols;
+  if (!zeroed) {
+    OCF_CUDA(cudaMemsetAsync(wl.state, 0, sizeof(int) * 2 * N, st));
+    OCF_CUDA(cudaMemsetAsync(wl.bits, 0, sizeof(uint32_t) * N * W, st));
   }
-  // rows that repeat a column: stream the store's CSC index (order-preserving compaction)
-  if (b->store->dev.n_groups == 0 || bt.n_entries == 0) return OCF_OK;
-  ColArgs a{};
-  a.s = b->store->dev; a.bt = bt;
-  a.n_cols = m->cfg.n_cols; a.nblk = m->nblk; a.bits = m->bits; a.dense = dense;
-  a.do_dec = do_dec; a.do_enc = do_enc;
-  a.err_flag = m->d_err; a.matches = wl.matches; a.mcol = wl.mcol; a.tasks = wl.tasks;
-  a.colseg = wl.seg; a.counters = wl.counters; a.max_matches = (int)m->cfg.max_entries;
-  const int64_t words = (b->store->n_rows + 31) / 32;
-  a.bitmap_words = words <= 40 * 1024 ? (int)words : 0;             // <= 160 KB of shared memory
-  const size_t smem = (size_t)a.bitmap_words * 4;
-  if (smem > 40 * 1024) OCF_CUDA(cudaFuncSetAttribute(k_col_scan, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int per_sm = (int)std::max<size_t>(1, std::min<size_t>(5, (200 * 1024) / std::max<size_t>(smem + 16 * 1024, 1)));
-  const int grid = std::max(1, std::min(m->sm_count * per_sm, b->store->dev.n_groups));
+  // a row that repeats a column merges its ratings into one record per (column, batch row): fields without a
+  // writer must read 0 (the whole capacity: a captured list graph serves every fill of the batch object)
+  if (dups) OCF_CUDA(cudaMemsetAsync(wl.matches, 0, sizeof(uint32_t) * 3 * (size_t)wl.entries, st));
+  SortArgs a{};
+  a.bt = bt;
+  a.cnt = wl.state; a.codeor = wl.state + N;
+  a.colinfo = wl.info; a.bits = wl.bits; a.W = W; a.counters = wl.counters;
+  a.matches = wl.matches; a.tasks = wl.tasks; a.colseg = wl.seg; a.heavy = heavy_model(m) ? wl.heavy : nullptr;
+  a.n_cols = m->cfg.n_cols; a.nblk = m->nblk; a.bits3 = m->bits; a.dense = dense; a.do_dec = do_dec; a.do_enc = do_enc;
+  a.dups = dups;
+  const int grid = item_grid(m, b);
   g_prof.begin(3, st);
-  k_col_scan<<<grid, 256, smem, st>>>(a);
+  k_sort_count<<<grid, 128, 0, st>>>(a);
+  OCF_LAUNCHED();
+  OCF_CUDA(launch_pdl(!g_prof.on, k_sort_alloc, dim3((m->cfg.n_cols + 255) / 256), dim3(256), st, a));
+  OCF_LAUNCHED();
+  OCF_CUDA(launch_pdl(!g_prof.on, k_sort_place, dim3(grid), dim3(128), st, a));
   OCF_LAUNCHED();
   g_prof.end(3, st);
   return OCF_OK;
@@ -1872,8 +1766,8 @@ static int launch_rows(ocf_model* m, const ocf_batch* b, int do_dec, int do_enc,
   r.matches = wl.matches; r.tasks = wl.tasks; r.colseg = wl.seg; r.counters = wl.counters;
   // small catalogues (weights + state within reach of the 126 MB L2): latency-bound, wide walk; else HBM-bound
   const bool wide = !grad_mode && (size_t)m->cfg.n_cols * (size_t)hpx <= ((size_t)8 << 20);
-  const bool heavy = heavy_model(m) && !b->store->has_dups && !grad_mode;      // exactly when K4a lists heavy tasks
-  r.heavy = heavy ? wl.heavy : nullptr;          // the batch-side K4a lists them; the CSC scan does not
+  const bool heavy = heavy_model(m) && !grad_mode;      // exactly when K4a lists heavy tasks
+  r.heavy = heavy ? wl.heavy : nullptr;
   r.hdec = drop ? m->h[L - 1] : m->act[L - 1]; r.dz0 = m->dz[0]; r.dy = m->dy;
   r.WdecT = dec.W; r.Wd_s1 = dec.Ws1; r.Wd_s2 = dec.Ws2; r.bdec = dec.b; r.bd_s1 = dec.bs1; r.bd_s2 = dec.bs2;
   r.Wenc = enc.W; r.We_s1 = enc.Ws1; r.We_s2 = enc.Ws2;
@@ -2181,7 +2075,7 @@ static int eval_body(ocf_model* m, ocf_batch* b, const ocf_step_args* args, cuda
 // enqueues a step or two ahead) instead of beside this step's K2 / K3.
 static bool ahead_ok(const ocf_model* m, const ocf_batch* b, const ocf_step_args* args) {
   return m->par_mode == 0 && m->comm == nullptr && (args == nullptr || args->phase == 0) && b->mode == 1 &&
-         b->store != nullptr && !b->store->has_dups && b->gathered_valid &&
+         b->store != nullptr && b->gathered_valid &&
          (m->layers[0].trainable || m->layers[m->L].trainable) && b->dev.B <= b->max_rows;
 }
 
@@ -2211,7 +2105,7 @@ static int worklist_alloc(ocf_batch* b, const ocf_model* m) {
   OCF_TRY(b->wl_mem.get(&b->wl.heavy, N * (size_t)(m->nblk + 1)));
   OCF_TRY(b->wl_mem.get(&b->wl.info, N));
   OCF_TRY(b->wl_mem.get(&b->wl.matches, (size_t)std::max<int64_t>(b->max_entries, 1) * 3));
-  b->wl.mcol = nullptr;
+  b->wl.entries = b->max_entries;
   b->wl_cols = m->cfg.n_cols; b->wl_nblk = m->nblk;
   return OCF_OK;
 }
@@ -2276,8 +2170,9 @@ static int run_step(ocf_model* m, ocf_batch* b, const ocf_step_args* args, bool 
   OCF_TRY(sync_step_state(m, args, st));
   auto body = [&](cudaStream_t s) { return train ? train_body(m, b, args, s) : eval_body(m, b, args, s); };
   bool done = false;
-  if (!g_prof.on && !b->store->has_dups) {
-    const auto key = std::make_tuple(b->uid, b->dev.B, train ? (wl_current(m, b) ? 3 : 1) : 0, args ? args->rows_total : 0, args ? args->row0 : 0);
+  if (!g_prof.on) {
+    const auto key = std::make_tuple(b->uid, b->dev.B, train ? (wl_current(m, b) ? 3 : 1) : 0, args ? args->rows_total : 0, args ? args->row0 : 0,
+                                     b->store->has_dups ? 1 : 0);
     ocf_model::StepGraph& g = m->graphs[key];
     if (g.exec == nullptr && !g.failed && g.seen++ >= 1) {
       const long long launched = g_launches.load();
@@ -2592,12 +2487,9 @@ extern "C" int ocf_model_read_metrics(ocf_model* m, int64_t first, int32_t count
   OCF_REQUIRE(count >= 0 && count <= LOG_CAP && first >= 0 && first + count <= m->steps_logged &&
               first + LOG_CAP >= m->steps_logged, "ocf_model_read_metrics: range not in the log");
   cudaStream_t st = as_stream(stream_);
-  int err = 0;
-  OCF_CUDA(cudaMemcpyAsync(&err, m->d_err, sizeof(int), cudaMemcpyDeviceToHost, st));
   OCF_CUDA(cudaStreamSynchronize(st));
   if (m->steps_logged > 0) OCF_CUDA(cudaEventSynchronize(m->step_ev[(m->steps_logged - 1) % 64]));
   for (int32_t k = 0; k < count; ++k)
     std::memcpy(host + (size_t)k * LOG_W, m->h_rec + (size_t)((first + k) % LOG_CAP) * LOG_W, sizeof(float) * LOG_W);
-  if (err != 0) return fail(OCF_ERR_STATE, "a catalogue column matched more batch entries than the update kernel's list holds (rows repeat a column too often)");
   return OCF_OK;
 }

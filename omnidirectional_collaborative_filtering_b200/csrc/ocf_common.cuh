@@ -49,8 +49,7 @@ constexpr uint8_t CODE_IN = 1;    // contributes ratings_batch_inputs / mask_bat
 constexpr uint8_t CODE_OBS = 2;   // contributes missing_data_mask
 constexpr uint8_t CODE_TGT = 4;   // contributes ratings_batch_targets / mask_batch_targets
 
-constexpr int SLOT_BITS = 12;             // rowslot = tag << 12 | batch row
-constexpr int MAX_BATCH_ROWS = 1 << SLOT_BITS;
+constexpr int MAX_BATCH_ROWS = 4096;
 constexpr int HPAD = 128;                 // hidden widths are padded to a multiple of 128 floats
 constexpr int MAX_HP = 1024;
 constexpr int ROWSTAT_W = 4;              // sse, sae, cnt, unused
@@ -61,14 +60,7 @@ struct StoreDev {
   const int32_t* col;
   const float* val;
   const int32_t* next_dup;   // index inside the row of the next later rating of the same column, or -1; null if no row repeats a column
-  const int64_t* colptr;     // CSC: entries of column c are [colptr[c], colptr[c+1])
-  const int32_t* crow;       //   row of the entry
-  const int32_t* cj;         //   position of the entry inside its row
-  const int32_t* ccol;       //   column of the entry (CSC expanded; read for matches only)
   const int32_t* orig_pos;   // column shards: position of the entry inside its FULL row (null: the store holds full rows)
-  const int2* groups;        //   scan schedule: groups of consecutive columns [x, y), <= scan_t entries each or one longer column; largest first
-  int n_groups;
-  int scan_t;                //   4096, 8192 or 16384: picked so that a scan is about one group per resident CTA
 };
 
 // What changes from one fill of a batch object to the next, as the device sees it: the first bytes of
@@ -79,7 +71,7 @@ struct BatchHdr {
   int B;
   int n_items;
   int n_entries;
-  uint32_t tag;              // rowslot tag of this fill
+  uint32_t pad0;
   int cdf_row0;              // device-RNG mode: index of batch row 0 among the drawing unit's sparsity draws
   int pass_through;
   double rng_lo, rng_range;  // np.random.uniform(lo, hi) of the rows' sparsity draws (range = hi - lo)
@@ -124,8 +116,6 @@ struct BatchDev {
   int32_t* ent_col;          // [n_entries]
   float* ent_val;            // [n_entries]
   uint8_t* codes;            // [n_entries]
-  uint32_t* rowslot;         // [store rows] tag << 12 | b for rows of this batch
-  uint32_t tag;
 };
 
 struct OptDev {

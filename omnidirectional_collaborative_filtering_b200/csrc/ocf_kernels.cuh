@@ -1,8 +1,7 @@
 // Hand-written sm_100a kernels of the training / scoring hot path.
 //
 // Data layout in HBM (DESIGN.md section 3):
-//   * rating store: CSR (rowptr i64, col i32, val f32); a CSC index (colptr i64, crow i32, cj i32)
-//     only for stores whose rows repeat a column
+//   * rating store: CSR (rowptr i64, col i32, val f32)
 //   * encoder kernel  Wenc  [k*N, HP]  (Keras layout, fan_out padded to a multiple of 128)
 //   * decoder kernel  WdecT [N, HP]    (TRANSPOSED Keras layout: one contiguous row per
 //     catalogue column, so the loss at an observed entry is one coalesced 4*HP-byte read)
@@ -43,7 +42,6 @@ k_gather_split(StoreDev s, BatchDev bt) {
   const int row = bt.row_ids[b];
   const int64_t src0 = s.rowptr[row];
   const int p0 = bt.ent_off[b];
-  if (start == 0 && threadIdx.x == 0 && bt.rowslot != nullptr) bt.rowslot[row] = (hd.tag << SLOT_BITS) | (uint32_t)b;
   const int d0 = RNG ? bt.draw_off[b] : 0;
   // the stream lives in a ring addressed by absolute position: word j of the batch's draws is ring word
   // (word_base + j) mod ring_words (a batch is shorter than the ring, so one conditional subtraction wraps)
@@ -763,213 +761,33 @@ k_dz_bias(const float* __restrict__ dh, const float* __restrict__ a, const float
 // ============================================================================================
 // K4: weight-side products fused with the optimizer update: a work list, then the update.
 //
-// (work list)  normally built from the batch alone by k_sort_* further down; for stores whose
-//              rows repeat a column by k_col_scan:
-// k_col_scan   streams the store's CSC row ids once. A CTA owns a group of consecutive catalogue
-//              columns (<= SCAN_T entries, or one longer column) and tests every entry's row
-//              against a shared-memory bitmap of the batch's rows. The matches (~1 % of the
-//              entries) are compacted IN CSC ORDER (ballot words + prefix sum, no sorting, no
-//              float atomics) into a global match list as (batch row, code, value, entry) records,
-//              so each column's matches are contiguous and deterministic. One task per weight row
-//              that must change is appended to a task list:
-//                array 0      decoder row  WdecT[c,:]  (+ b_dec[c])   needs a target entry
-//                array 1+blk  encoder row  Wenc[blk*N+c,:]            needs an entry with the block's bit
-//              With a dense rule (RMSprop / Adam / L2) every row changes: the scan only records
-//              each touched column's segment and the update enumerates all (column, array) pairs.
-// k_row_update one warp per task, persistent grid: issue the loads of the weight row and its
+// K4a (k_sort_*) groups the batch's own ratings by catalogue column with a counting sort over the
+// ~10^5 gathered entries:
+//   count   per entry: the column's count of matched batch rows, the OR of its code bits (int atomics) and
+//           bit `batch row` of the column's row of the presence bitmap [n_cols][W words]
+//   alloc   per COLUMN (a coalesced sweep over the count array): a touched column reserves its segment of
+//           the match list and its update tasks; one atomic per warp and counter (warp-aggregated), and
+//           the tasks come out in column order inside a warp: neighbouring tasks touch neighbouring
+//           weight rows. One task per weight row that must change:
+//             array 0      decoder row  WdecT[c,:]  (+ b_dec[c])   needs a target entry
+//             array 1+blk  encoder row  Wenc[blk*N+c,:]            needs an entry with the block's bit
+//           With a dense rule (RMSprop / Adam / L2) every row changes: alloc also records each touched
+//           column's segment and the update enumerates all (column, array) pairs.
+//   place   per entry: rank inside its column = popcount of the lower batch rows present, so a column's
+//           matches are ordered by batch row whatever order the atomics ran in: the gradient sums of K4b
+//           keep a fixed order (bit-reproducible steps)
+// A match record is one (batch row, column) cell: (batch row | code << 16, value, entry index). When a
+// row repeats a column (`dups`), the cell's ratings share one record: K1's code bits give each array
+// exactly one live writer per cell (the reference's dense arrays are last-write-wins), so the record
+// ORs the codes of the cell's entries and takes the value from the CODE_IN writer and the entry index
+// (-> dy) from the CODE_TGT writer; the list is zeroed first, so a field without a writer reads 0.
+// Three small kernels beside K2 / K3 on a low-priority stream, or ahead of the step on the batch's.
+//
+// K4b (k_row_update) one warp per task, persistent grid: issue the loads of the weight row and its
 //              optimizer state, accumulate the gradient from the matched activations
 //                decoder:  g = sum_b dy[b,c] * h[b,:]        encoder:  g = sum_b x0[b,blk*N+c] * dz[b,:]
 //              in registers, apply the update, store. W and state are read once and written once
 //              (16 B/param for Adagrad/RMSprop, 24 for Adam), only for rows that change.
-// ============================================================================================
-constexpr int SCAN_SUB = 4096;            // CSC entries per sub-block (256 threads x 16 loads in flight)
-constexpr int SCAN_T_MAX = 16384;         // largest scan block (a store picks 4096, 8192 or 16384)
-constexpr int SCAN_WORDS_MAX = SCAN_T_MAX / 32;
-constexpr int SCAN_STAGE = 2048;          // matches of one group staged in shared memory for task creation
-
-struct ColArgs {
-  StoreDev s; BatchDev bt;
-  int n_cols; int nblk; int3 bits; int dense; int do_dec; int do_enc;
-  int* err_flag;
-  uint32_t* matches;      // [max_entries * 3]  b | code << 16, value bits, batch entry index (-> dy)
-  int32_t* mcol;          // [max_entries]      catalogue column of the match
-  int4* tasks;            // sparse rules: (column, array, first match, match count)
-  int2* colseg;           // dense rules:  per column (first match, match count), zeroed per step
-  int* counters;          // [0] matches used, [1] tasks
-  int bitmap_words;       // 32-bit words of the shared-memory row bitmap (0: too many rows, skip it)
-  int max_matches;
-};
-
-__global__ void __launch_bounds__(256) k_col_scan(ColArgs a) {
-  extern __shared__ uint32_t col_smem[];
-  __shared__ uint32_t words[SCAN_WORDS_MAX];
-  __shared__ int prefix[SCAN_WORDS_MAX + 1];
-  __shared__ int s_base, s_tbase;
-  __shared__ int s_wsum[8];
-  __shared__ int s_mc[SCAN_STAGE];
-  __shared__ uint8_t s_code[SCAN_STAGE];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int T = a.s.scan_t, nwords = T / 32;
-  uint32_t* bitmap = col_smem;
-  if (a.bitmap_words > 0) {
-    for (int i = threadIdx.x; i < a.bitmap_words; i += blockDim.x) bitmap[i] = 0u;
-    __syncthreads();
-    for (int i = threadIdx.x; i < a.bt.hdr->B; i += blockDim.x) {
-      const int r = a.bt.row_ids[i];
-      atomicOr(&bitmap[r >> 5], 1u << (r & 31));
-    }
-    __syncthreads();
-  }
-  for (int g = blockIdx.x; g < a.s.n_groups; g += gridDim.x) {
-    const int2 grp = a.s.groups[g];
-    const int64_t e0 = a.s.colptr[grp.x], e1 = a.s.colptr[grp.y];
-    const int nblocks = (int)((e1 - e0 + T - 1) / T);
-
-    // phase 1 of a block: match bit of every entry -> words[], exclusive prefix of the word
-    // popcounts -> prefix[], block total -> prefix[nwords]
-    auto find = [&](int64_t eb) {
-      const int lim = (int)min((int64_t)T, e1 - eb);          // entries of this block
-      const int32_t* cr = a.s.crow + eb;
-      for (int sb = 0; sb < T / SCAN_SUB; ++sb) {
-        int row[16];
-        const int off0 = sb * SCAN_SUB + warp * 32 + lane;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) row[i] = off0 + i * 256 < lim ? cr[off0 + i * 256] : -1;
-#pragma unroll
-        for (int i = 0; i < 16; ++i) {
-          // the bitmap holds exactly this batch's rows, so membership needs no global lookup;
-          // only stores with too many rows for shared memory fall back to the row -> slot map
-          bool match = row[i] >= 0;
-          if (match) match = a.bitmap_words > 0 ? ((bitmap[row[i] >> 5] >> (row[i] & 31)) & 1u) != 0
-                                                : (a.bt.rowslot[row[i]] >> SLOT_BITS) == a.bt.hdr->tag;
-          const unsigned m = __ballot_sync(FULL, match);
-          if (lane == 0) words[sb * (SCAN_SUB / 32) + warp + 8 * i] = m;
-        }
-      }
-      __syncthreads();
-      if (warp == 0) {
-        int run = 0;
-        for (int k = 0; k < nwords / 32; ++k) {
-          const int cnt = __popc(words[k * 32 + lane]);
-          int inc = cnt;
-#pragma unroll
-          for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(FULL, inc, o); if (lane >= o) inc += t; }
-          prefix[k * 32 + lane] = run + inc - cnt;
-          run += __shfl_sync(FULL, inc, 31);
-        }
-        if (lane == 0) prefix[nwords] = run;
-      }
-      __syncthreads();
-    };
-
-    int total = 0;
-    if (nblocks == 1) { find(e0); total = prefix[nwords]; }
-    else for (int blk = 0; blk < nblocks; ++blk) { find(e0 + (int64_t)blk * T); total += prefix[nwords]; __syncthreads(); }
-    if (total == 0) continue;
-    if (threadIdx.x == 0) {
-      const int got = atomicAdd(&a.counters[0], total);
-      if (got + total > a.max_matches) { atomicExch(a.err_flag, 1); s_base = -1; } else s_base = got;
-    }
-    __syncthreads();
-    const int base = s_base;
-    if (base < 0) continue;
-    int running = 0;
-    for (int blk = 0; blk < nblocks; ++blk) {
-      const int64_t eb = e0 + (int64_t)blk * T;
-      if (nblocks > 1) find(eb);
-      // phase 2: one thread per match (their dependent load chains run side by side): locate the
-      // t-th set bit of the block, fetch the batch record, write it at CSC rank base+running+t
-      const int block_total = prefix[nwords];
-      for (int t = threadIdx.x; t < block_total; t += blockDim.x) {
-        int wlo = 0, whi = nwords;
-        while (whi - wlo > 1) { const int mid = (wlo + whi) >> 1; if (prefix[mid] <= t) wlo = mid; else whi = mid; }
-        const int bitpos = __fns(words[wlo], 0, t - prefix[wlo] + 1);
-        const int64_t e = eb + wlo * 32 + bitpos;
-        const uint32_t b = a.bt.rowslot[a.s.crow[e]] & (uint32_t)(MAX_BATCH_ROWS - 1);
-        const int p = a.bt.ent_off[b] + a.s.cj[e];
-        const size_t idx = (size_t)(base + running + t);
-        a.matches[idx * 3] = b | ((uint32_t)a.bt.codes[p] << 16);
-        a.matches[idx * 3 + 1] = __float_as_uint(a.bt.ent_val[p]);
-        a.matches[idx * 3 + 2] = (uint32_t)p;   // the scan needs nothing of the forward pass: it runs beside it
-        a.mcol[idx] = a.s.ccol[e];
-      }
-      running += block_total;
-      __syncthreads();
-    }
-    // phase 3: one head per column segment creates that column's tasks. Task slots are
-    // allocated with ONE atomic per 256 matches (block scan of the per-head task counts):
-    // per-column atomics on a single counter serialise in L2 and dominated this kernel.
-    // (the group's match columns / codes are staged in shared memory first: a head thread walks
-    // its segment there; walking a heavy column's ~B matches through L2 was this kernel's tail)
-    const bool staged = total <= SCAN_STAGE;
-    if (staged) {
-      for (int i = threadIdx.x; i < total; i += blockDim.x) {
-        s_mc[i] = __ldcg(a.mcol + base + i);
-        s_code[i] = (uint8_t)(__ldcg(a.matches + (size_t)(base + i) * 3) >> 16);
-      }
-      __syncthreads();
-    }
-    for (int i0 = 0; i0 < total; i0 += blockDim.x) {
-      const int i = i0 + threadIdx.x;
-      int c = -1, n = 0, n_tasks = 0;
-      int arr[4];
-      if (i < total) {
-        uint32_t any_code = 0;
-        bool head;
-        if (staged) {
-          c = s_mc[i];
-          head = i == 0 || s_mc[i - 1] != c;
-          if (head) while (i + n < total && s_mc[i + n] == c) { any_code |= s_code[i + n]; ++n; }
-        } else {
-          c = __ldcg(a.mcol + base + i);
-          head = i == 0 || __ldcg(a.mcol + base + i - 1) != c;
-          if (head) while (i + n < total && __ldcg(a.mcol + base + i + n) == c) { any_code |= __ldcg(a.matches + (size_t)(base + i + n) * 3) >> 16; ++n; }
-        }
-        if (head) {
-          if (a.dense) a.colseg[c] = make_int2(base + i, n);
-          else {
-            if (a.do_dec && (any_code & CODE_TGT)) arr[n_tasks++] = 0;
-            if (a.do_enc)
-              for (int blk = 0; blk < a.nblk; ++blk) {
-                const int bit = blk == 0 ? a.bits.x : (blk == 1 ? a.bits.y : a.bits.z);
-                if (any_code & bit) arr[n_tasks++] = 1 + blk;
-              }
-          }
-        }
-      }
-      if (a.dense) continue;
-      int inc = n_tasks;
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) { const int t = __shfl_up_sync(FULL, inc, o); if (lane >= o) inc += t; }
-      if (lane == 31) s_wsum[warp] = inc;
-      __syncthreads();
-      if (threadIdx.x == 0) {
-        int tot = 0;
-        for (int w2 = 0; w2 < 8; ++w2) { const int t = s_wsum[w2]; s_wsum[w2] = tot; tot += t; }
-        s_tbase = tot > 0 ? atomicAdd(&a.counters[1], tot) : 0;
-      }
-      __syncthreads();
-      const int slot = s_tbase + s_wsum[warp] + inc - n_tasks;
-      for (int k = 0; k < n_tasks; ++k) a.tasks[slot + k] = make_int4(c, arr[k], base + i, n);
-      __syncthreads();
-    }
-  }
-}
-
-// ============================================================================================
-// K4a, batch-side: groups the batch's own ratings by catalogue column with a counting sort over
-// the ~10^5 gathered entries instead of streaming the store's CSC index (10^7-10^8 entries):
-//   count   per entry: the column's live-entry count, the OR of its code bits (int atomics) and bit
-//           `batch row` of the column's row of the presence bitmap [n_cols][W words]
-//   alloc   per COLUMN (a coalesced sweep over the count array): a touched column reserves its segment of
-//           the match list and its update tasks; one atomic per warp and counter (warp-aggregated), and
-//           the tasks come out in column order inside a warp: neighbouring tasks touch neighbouring
-//           weight rows
-//   place   per entry: rank inside its column = popcount of the lower batch rows present, so a column's
-//           matches are ordered by batch row whatever order the atomics ran in: the gradient sums of K4b
-//           keep a fixed order (bit-reproducible steps)
-// A (column, batch row) pair is unique unless a row repeats a column; stores with repeats keep
-// using the CSC scan above. Three small kernels beside K2 / K3 on a low-priority stream.
 // ============================================================================================
 struct SortArgs {
   BatchDev bt;
@@ -980,6 +798,7 @@ struct SortArgs {
   uint32_t* matches; int4* tasks; int2* colseg;
   int4* heavy;                              // (column, array, first match, matches) of every task with more than HEAVY_N matches (null: none recorded)
   int n_cols; int nblk; int3 bits3; int dense; int do_dec; int do_enc;
+  int dups;                                 // some row of the store repeats a column: one match per (column, batch row), list zeroed
 };
 
 __global__ void __launch_bounds__(128) k_sort_count(SortArgs a) {
@@ -990,9 +809,16 @@ __global__ void __launch_bounds__(128) k_sort_count(SortArgs a) {
     const int code = a.bt.codes[p0 + i];
     if (code == 0) continue;
     const int c = a.bt.ent_col[p0 + i];
-    atomicAdd(&a.cnt[c], 1);
-    atomicOr(&a.codeor[c], code);
-    atomicOr(&a.bits[(size_t)c * a.W + (b >> 5)], 1u << (b & 31));
+    if (a.dups) {
+      // the first of the row's ratings of this column to set its bit counts the row
+      const uint32_t bit = 1u << (b & 31);
+      if ((atomicOr(&a.bits[(size_t)c * a.W + (b >> 5)], bit) & bit) == 0u) atomicAdd(&a.cnt[c], 1);
+      atomicOr(&a.codeor[c], code);
+    } else {
+      atomicAdd(&a.cnt[c], 1);
+      atomicOr(&a.codeor[c], code);
+      atomicOr(&a.bits[(size_t)c * a.W + (b >> 5)], 1u << (b & 31));
+    }
   }
 }
 
@@ -1071,9 +897,16 @@ __global__ void __launch_bounds__(128) k_sort_place(SortArgs a) {
     int rank = __popc(bw[b >> 5] & ((1u << (b & 31)) - 1u));
     for (int w = 0; w < (b >> 5); ++w) rank += __popc(bw[w]);
     const size_t idx = (size_t)(info.x + rank);
-    a.matches[idx * 3] = (uint32_t)b | (code << 16);
-    a.matches[idx * 3 + 1] = __float_as_uint(a.bt.ent_val[p]);
-    a.matches[idx * 3 + 2] = (uint32_t)p;
+    if (a.dups) {
+      // the row's ratings of this column share the record; each field has at most one writer
+      atomicOr(&a.matches[idx * 3], (uint32_t)b | (code << 16));
+      if (code & CODE_IN) a.matches[idx * 3 + 1] = __float_as_uint(a.bt.ent_val[p]);
+      if (code & CODE_TGT) a.matches[idx * 3 + 2] = (uint32_t)p;
+    } else {
+      a.matches[idx * 3] = (uint32_t)b | (code << 16);
+      a.matches[idx * 3 + 1] = __float_as_uint(a.bt.ent_val[p]);
+      a.matches[idx * 3 + 2] = (uint32_t)p;
+    }
   }
 }
 

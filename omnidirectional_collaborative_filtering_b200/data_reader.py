@@ -517,7 +517,7 @@ class data_reader(object):
                     raw = self.densevec_to_users[i]
                     lists.append(user_dict[raw] if raw in user_dict else user_dict[str(raw)])
                 csr = _csr_from_lists(lists, self.items_to_densevec, N)
-            self._stores["train"] = RatingStore(csr, build_csc=True)
+            self._stores["train"] = RatingStore(csr)
         elif native:
             # the three files parse concurrently (ctypes releases the GIL inside the library)
             from concurrent.futures import ThreadPoolExecutor
@@ -528,7 +528,7 @@ class data_reader(object):
                 self.val_set, va_in, _, va_tg = jobs[1].result()
                 self.test_set, te_in, _, te_tg = jobs[2].result()
             self._set_sizes()
-            self._stores["train"] = RatingStore(train, build_csc=True)
+            self._stores["train"] = RatingStore(train)
             self._stores["valid"] = StorePair(RatingStore(va_in), RatingStore(va_tg))
             self._stores["test"] = StorePair(RatingStore(te_in), RatingStore(te_tg))
         else:
@@ -540,7 +540,7 @@ class data_reader(object):
             self.test_set = list(test[1].keys())
             self._set_sizes()
             col_of = self.items_to_densevec
-            self._stores["train"] = RatingStore(_csr_from_lists(list(train.values()), col_of, N), build_csc=True)
+            self._stores["train"] = RatingStore(_csr_from_lists(list(train.values()), col_of, N))
             for name, (ins, tgs), keys in (("valid", valid, self.val_set), ("test", test, self.test_set)):
                 pair = StorePair(RatingStore(_csr_from_lists([ins[k] for k in keys], col_of, N)),
                                  RatingStore(_csr_from_lists([tgs[k] for k in keys], col_of, N)))
@@ -565,7 +565,7 @@ class data_reader(object):
         self.val_set, va_in, _, va_tg = ls.valid
         self.test_set, te_in, _, te_tg = ls.test
         self._set_sizes()
-        self._stores["train"] = RatingStore(widen(train), build_csc=True)
+        self._stores["train"] = RatingStore(widen(train))
         self._stores["valid"] = StorePair(RatingStore(widen(va_in)), RatingStore(widen(va_tg)))
         self._stores["test"] = StorePair(RatingStore(widen(te_in)), RatingStore(widen(te_tg)))
 
@@ -584,7 +584,7 @@ class data_reader(object):
         self.val_set = [str(int(k)) for k in fs.valid_keys]
         self.test_set = [str(int(k)) for k in fs.test_keys]
         self.train_set_size, self.val_set_size, self.test_set_size = len(self.train_set), len(self.val_set), len(self.test_set)
-        self._stores["train"] = RatingStore(fs.train, build_csc=True)
+        self._stores["train"] = RatingStore(fs.train)
         self._stores["valid"] = StorePair(RatingStore(fs.valid_in), RatingStore(fs.valid_tg))
         self._stores["test"] = StorePair(RatingStore(fs.test_in), RatingStore(fs.test_tg))
 

@@ -12,11 +12,10 @@ from .synthetic import Csr
 
 class RatingStore(object):
     """One set of per-row rating lists (what `data_reader.py:46-70` keeps as dicts) as CSR on
-    the host, uploaded to HBM on first use. `build_csc` adds the column index training needs."""
+    the host, uploaded to HBM on first use."""
 
-    def __init__(self, csr: Csr, build_csc: bool = False, orig_pos=None, full_lengths=None):
+    def __init__(self, csr: Csr, orig_pos=None, full_lengths=None):
         self.csr = csr
-        self.build_csc = bool(build_csc)
         self._handle = None
         # column shards (dist.py): position of each kept rating inside its full row, and the full
         # row lengths (the RNG replay and target counts are defined on full rows)
@@ -51,7 +50,7 @@ class RatingStore(object):
         rowptr = np.zeros(c.n_rows + 1, dtype=np.int64)
         np.cumsum(np.bincount(rows[keep], minlength=c.n_rows), out=rowptr[1:])
         local = Csr(c.n_rows, hi - lo, rowptr, (c.col[keep] - lo).astype(np.int32), c.val[keep].copy())
-        return RatingStore(local, self.build_csc, orig_pos=pos[keep].astype(np.int32), full_lengths=self.lengths)
+        return RatingStore(local, orig_pos=pos[keep].astype(np.int32), full_lengths=self.lengths)
 
     @property
     def handle(self):
@@ -62,8 +61,7 @@ class RatingStore(object):
             val = np.ascontiguousarray(self.csr.val, dtype=np.float32)
             out = C.c_void_p()
             _lib.check(_lib.lib().ocf_store_create(self.csr.n_rows, self.csr.n_cols, _lib.ptr(rowptr),
-                                                   _lib.ptr(col), _lib.ptr(val), int(self.build_csc),
-                                                   C.byref(out)))
+                                                   _lib.ptr(col), _lib.ptr(val), C.byref(out)))
             self._handle = out
             if self.orig_pos is not None:
                 op = np.ascontiguousarray(self.orig_pos, dtype=np.int32)
@@ -71,9 +69,9 @@ class RatingStore(object):
         return self._handle
 
     def info(self):
-        buf = (C.c_int64 * 6)()
+        buf = (C.c_int64 * 5)()
         _lib.check(_lib.lib().ocf_store_info(self.handle, buf))
-        return dict(zip(("n_rows", "n_cols", "nnz", "has_dups", "max_col_len", "device_bytes"), list(buf)))
+        return dict(zip(("n_rows", "n_cols", "nnz", "has_dups", "device_bytes"), list(buf)))
 
     def close(self):
         if self._handle is not None:

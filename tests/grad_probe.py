@@ -83,6 +83,15 @@ def from_dense(feed, targets, aux_type):
     return SparseBatch(mask.shape[0], mask.shape[1], len(parts), x0, r, c, t[r, c], mask[r, c])
 
 
+def _last_writes(r, c, v, width):
+    """The last of the writes (r, c, v) to each cell (r, c) of a [*, width] array: the dense fills are
+    last-write-wins, so a row that repeats a column keeps one value per array."""
+    key = (r * width + c)[::-1]
+    _, first = np.unique(key, return_index=True)
+    keep = r.size - 1 - first
+    return r[keep], c[keep], v[keep]
+
+
 def from_batch(batch):
     """SparseBatch of a product `data_reader.Batch` of kind "split" (restates data_reader.py:158-169 on arrays;
     the keep flags must be host-drawn: a reader with rng_on_device = False)."""
@@ -105,9 +114,11 @@ def from_batch(batch):
         ri.append(b); ci.append(c + blk * N); vi.append(np.full(b.size, a))      # observed
     if aux in ("dropout", "both"):
         ri.append(b[f]); ci.append(c[f] + N); vi.append(np.full(int(f.sum()), a))  # mask_in
-    x0 = sp.csr_matrix((np.concatenate(vi), (np.concatenate(ri), np.concatenate(ci))), shape=(B, nblk * N))
+    xr, xc, xv = _last_writes(np.concatenate(ri), np.concatenate(ci), np.concatenate(vi), nblk * N)
+    x0 = sp.csr_matrix((xv, (xr, xc)), shape=(B, nblk * N))
     tg = ~f | bool(batch.pass_through)
-    return SparseBatch(B, N, nblk, x0, b[tg], c[tg], v[tg], np.full(int(tg.sum()), a))
+    tr, tc, tv = _last_writes(b[tg], c[tg], v[tg], N)
+    return SparseBatch(B, N, nblk, x0, tr, tc, tv, np.full(tr.size, a))
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -358,16 +369,16 @@ def pad(h):
     return -(-int(h) // HPAD) * HPAD
 
 
-def row_launches(n_cols, widths, kind, has_dups=False, row_parallel=False):
+def row_launches(n_cols, widths, kind, row_parallel=False):
     """(NV, KIND, WIDE, HEAVY) of every k_row_update launch of one training step, mirroring
         wide  = !grad_mode && n_cols * hp_of_the_launch <= 8 Mi                   (launch_rows)
-        heavy = n_cols * max(hp[0], hp[L-1]) <= 32 Mi && !has_dups && !grad_mode  (heavy_model, launch_rows)
+        heavy = n_cols * max(hp[0], hp[L-1]) <= 32 Mi && !grad_mode                (heavy_model, launch_rows)
         WIDE launches the <NV, KIND, true, true> kernel (launch_row_update)
     and one launch when the decoder and encoder rows share a padded width, else one per width (phase_update).
     Row-parallel steps launch <NV, KIND_GRAD, false, false>. NV = hp / 128 capped at 8 (OCF_NV_SWITCH)."""
     hp0, hpt = pad(widths[0]), pad(widths[-1])
     grad = bool(row_parallel)
-    heavy = n_cols * max(hp0, hpt) <= (32 << 20) and not has_dups and not grad
+    heavy = n_cols * max(hp0, hpt) <= (32 << 20) and not grad
     out = []
     for hp in sorted({hpt, hp0}):
         nv = min(hp // 128, 8)

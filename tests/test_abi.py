@@ -16,7 +16,7 @@ def test_library_exports_every_declared_symbol():
     for name in names:
         assert hasattr(lib, name), "include/ocf.h declares %s but libocf_b200.so does not export it" % name
     assert set(names) == set(_lib._SIGNATURES), "ctypes signatures out of sync with include/ocf.h"
-    assert lib.ocf_version() == 100
+    assert lib.ocf_version() == 101
 
 
 def test_exports_are_plain_c():
@@ -35,7 +35,7 @@ def test_argument_validation_needs_no_gpu():
     out = C.c_void_p()
     rowptr = np.array([0, 2, 1], dtype=np.int64)           # not monotone
     col = np.zeros(2, dtype=np.int32); val = np.zeros(2, dtype=np.float32)
-    st = lib.ocf_store_create(2, 4, _lib.ptr(rowptr), _lib.ptr(col), _lib.ptr(val), 0, C.byref(out))
+    st = lib.ocf_store_create(2, 4, _lib.ptr(rowptr), _lib.ptr(col), _lib.ptr(val), C.byref(out))
     assert st == -1 and b"monotone" in lib.ocf_last_error()
     cfg = _lib.ModelConfig()
     cfg.n_cols = 10; cfg.n_cols_total = 10; cfg.n_layers = 0

@@ -97,9 +97,9 @@ def _store(n_cols, B, seed):
 class Cell(object):
     """A store, its one stepped batch and a model over it."""
 
-    def __init__(self, widths, n_cols, B, aux, act, loss, pdrop, pt=False, seed=0):
+    def __init__(self, widths, n_cols, B, aux, act, loss, pdrop, pt=False, seed=0, store=_store):
         self.widths, self.n_cols, self.B, self.aux, self.act, self.loss, self.pdrop = widths, n_cols, B, aux, act, loss, pdrop
-        fs, self.special = _store(n_cols, B, seed)
+        fs, self.special = store(n_cols, B, seed)
         self.rd = data_reader(n_cols, B, "", eval_mode="fixed_split", data=fs, rng_on_device=False)
         np.random.seed(seed + 1)
         self.batch = next(self.rd.data_gen(B, SPARSITY, "train", False, aux, A, pass_through_input_training=pt))
@@ -240,6 +240,16 @@ def test_eager_captured_and_replayed_steps_agree(capfd):
     """The same SGD step from the same weights on one device batch: plain launches, then captured into a CUDA
     graph, then replayed. The weights it leaves are bit-identical, and each is inside the probe's bound."""
     c = Cell([300], n_cols_for("heavy", 384), 257, "causal", "sigmoid", "mean_squared_error", None, seed=5)
+    try:
+        check_graph_steps(c, capfd)
+    finally:
+        c.close()
+
+
+def check_graph_steps(c, capfd):
+    """Runs one SGD step of cell `c` three times from the same weights on one device batch (eager, captured,
+    replayed) and checks the weights each leaves against the probe and against each other, bit for bit. The cell has
+    no dropout: run k is step k, and the probe's reference is the step-0 one."""
     old = os.environ.get("OCF_DEBUG_GRAPH")
     os.environ["OCF_DEBUG_GRAPH"] = "1"
     try:
@@ -270,7 +280,6 @@ def test_eager_captured_and_replayed_steps_agree(capfd):
             os.environ.pop("OCF_DEBUG_GRAPH", None)
         else:
             os.environ["OCF_DEBUG_GRAPH"] = old
-        c.close()
 
 
 def test_cells_reach_every_instantiation():

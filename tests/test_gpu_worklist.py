@@ -6,7 +6,8 @@
   encoder rows leave and re-enter it);
 * the same steps with the grouping inside the step (a step driven phase by phase keeps it there) and ahead of it:
   bit-identical weights.
-Against the NumPy oracle on the same batches (reference: model.py:34-99, train.py:50-51)."""
+Against the NumPy oracle on the same batches (reference: model.py:34-99, train.py:50-51). The golden "rev" train store
+repeats columns inside rows (asserted in `_streams`), so these steps also cover the list's merged match records."""
 import ctypes as C
 
 import numpy as np
@@ -22,6 +23,7 @@ pytestmark = pytest.mark.gpu
 
 def _streams(ds, aux, pt, seed=3, B=8):
     rd = product_reader(ds, "fixed_split")
+    assert rd.store("train").info()["has_dups"] == 1
     data = oracle_data(ds, "fixed_split")
     np.random.seed(seed)
     gen = rd.data_gen(B, [0.2, 0.9], "train", True, aux, -1, pass_through_input_training=pt)

@@ -5,6 +5,7 @@ import pytest
 
 from oracle import ref_batches, ref_model
 from tests import grad_probe as gp
+from tests.helpers import oracle_data, product_reader
 
 A = 0.5          # a non-unit aux_var_value
 
@@ -193,6 +194,38 @@ def test_rule_probe_rejects_rmsprop_state_read_as_zero():
     assert fails and all(f.startswith("step 2") for f in fails), fails
 
 
+@pytest.mark.parametrize("pt", [False, True], ids=["split", "pass-through"])
+@pytest.mark.parametrize("aux", [None, "causal", "dropout", "zeros", "both"])
+def test_from_batch_keeps_last_write_of_repeated_columns(golden_datasets, aux, pt):
+    """`from_batch` of the product's batches equals `from_dense` of the oracle's dense batches on a store whose rows
+    repeat columns: one value per (row, column, array), the last write's (data_reader.py:158-169)."""
+    ds = golden_datasets["rev"]
+    rd = product_reader(ds, "fixed_split")
+    rd.rng_on_device = False          # host stream where a GPU exists too: the oracle replays it
+    np.random.seed(3)
+    gen = rd.data_gen(8, [0.2, 0.9], "train", True, aux, -1, pass_through_input_training=pt)
+    rgen = ref_batches.batch_stream(oracle_data(ds, "fixed_split"), 8, [0.2, 0.9], "train", True, aux, -1,
+                                    pass_through_input_training=pt, rng=np.random.RandomState(3))
+    repeats = 0
+    while True:
+        batch = next(gen)
+        if batch is None:
+            break
+        csr = batch.source.csr
+        for r in batch.rows:
+            cols, _ = csr.row(int(r))
+            repeats += len(cols) - np.unique(cols).size
+        feed, targets = next(rgen)
+        got, want = gp.from_batch(batch), gp.from_dense(feed, targets, aux)
+        assert (got.B, got.N, got.nblk) == (want.B, want.N, want.nblk)
+        assert np.array_equal(got.x0.toarray(), want.x0.toarray())
+        og, ow = np.lexsort((got.t_col, got.t_row)), np.lexsort((want.t_col, want.t_row))
+        for name in ("t_row", "t_col", "t_val", "t_mask"):
+            assert np.array_equal(getattr(got, name)[og], getattr(want, name)[ow]), name
+    assert repeats > 0                 # the batches did hold rows that repeat a column
+    rd.close()
+
+
 def test_variant_classifier_thresholds():
     M = 1 << 20
     # one width: WIDE up to n_cols * hp = 8 Mi, then HEAVY up to 32 Mi, then lean
@@ -202,8 +235,8 @@ def test_variant_classifier_thresholds():
     assert gp.row_launches(262145, [128], "sgd") == [(1, 0, False, False)]
     assert gp.row_launches(8 * M // 1024, [1000], "adam") == [(8, 3, True, True)]
     assert gp.row_launches(32 * M // 1024 + 1, [1024], "rmsprop") == [(8, 2, False, False)]
-    assert gp.row_launches(32769, [1024], "adam", has_dups=True) == [(8, 3, False, False)]
-    assert gp.row_launches(8192, [1024], "adam", has_dups=True) == [(8, 3, True, True)]
+    assert gp.row_launches(32769, [1024], "adam") == [(8, 3, False, False)]
+    assert gp.row_launches(8192, [1024], "adam") == [(8, 3, True, True)]
     # two ends of a width list: one launch per padded width, HEAVY decided by the wider end
     assert gp.row_launches(40000, [1024, 100], "sgd") == [(1, 0, True, True), (8, 0, False, False)]
     assert gp.row_launches(20000, [1024, 130], "sgd") == [(2, 0, True, True), (8, 0, False, True)]
