@@ -262,6 +262,15 @@ int ocf_score(ocf_model* model, ocf_batch* batch, float* out, int out_is_device,
  * hold column -1 / score -inf. Column shards return their own columns' top k (local ids). */
 int ocf_score_topk(ocf_model* model, ocf_batch* batch, int32_t k, int exclude_inputs,
                    int32_t* out_cols, float* out_scores, void* stream);
+/* Ranking evaluation on top of ocf_score (see DESIGN): for every batch entry that is a relevant
+ * target, its 1-based rank among the row's candidate columns (score desc, column asc: the order of
+ * ocf_score_topk). exclude_inputs != 0 removes the row's input columns from the candidates and from the
+ * relevant set; min_value: targets with a stored value below it are not relevant (-INFINITY = all).
+ * out_col[e], out_rank[e] for e < ocf_batch_info()[1] entries (rank 0 = not a relevant target),
+ * out_row_ptr[rows + 1] = the rows' entry ranges, out_n_cand[rows]. Synchronises `stream`. */
+int ocf_rank_targets(ocf_model* model, ocf_batch* batch, int exclude_inputs, float min_value,
+                     int32_t* out_col, int32_t* out_rank, int32_t* out_row_ptr, int64_t* out_n_cand,
+                     void* stream);
 /* The dense contraction kernel of the training step (tcgen05 kind::tf32 with fp32 operands split hi/lo, TMEM
  * accumulators, split-K over a thread-block cluster reduced through distributed shared memory;
  * csrc/ocf_gemm_tc.cuh: hidden layers of model.py:64-71 forward / backward / weight gradient), on host arrays:
@@ -389,7 +398,8 @@ int ocf_split_destroy(ocf_split* split);
 /* Per-kernel timing with CUDA events recorded on the launching stream around the named kernels
  * (tag 0 = K1 gather, 1 = K2 encoder, 2 = K3 decoder/loss, 3 = K4a column scan, 4 = scoring GEMM,
  * 5 = K4b row update, 6 = first collective of a parallel step (z all-reduce / streaming optimizer
- * pass), 7 = second collective (row statistics + dL/dh all-reduce / gradient all-reduce)). Off by default; ocf_profile_read synchronises the device and sums the elapsed times
+ * pass), 7 = second collective (row statistics + dL/dh all-reduce / gradient all-reduce), 9 = ranking
+ * evaluation kernels of ocf_rank_targets). Off by default; ocf_profile_read synchronises the device and sums the elapsed times
  * of the launches recorded since the last reset. */
 int ocf_profile_enable(int on);
 int ocf_profile_reset(void);

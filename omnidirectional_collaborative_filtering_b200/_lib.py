@@ -108,6 +108,7 @@ _SIGNATURES = {
     "ocf_predict": (C.c_int, [_P, _P, _P, _P]),
     "ocf_score": (C.c_int, [_P, _P, _P, C.c_int, _P]),
     "ocf_score_topk": (C.c_int, [_P, _P, C.c_int32, C.c_int, _P, _P, _P]),
+    "ocf_rank_targets": (C.c_int, [_P, _P, C.c_int, C.c_float, _P, _P, _P, _P, _P]),
     "ocf_gemm_tc": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, _P]),
     "ocf_gemm_tc_profile": (C.c_int, [C.c_int, C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int, C.c_int, C.c_int,
                                       C.POINTER(C.c_float), C.POINTER(C.c_int64)]),

@@ -17,6 +17,7 @@
 #include "ocf_score_tc.cuh"
 #include "ocf_gemm_tc.cuh"
 #include "ocf_topk.cuh"
+#include "ocf_rank.cuh"
 
 namespace ocf {
 
@@ -273,6 +274,12 @@ struct ocf_model {
   int32_t* topk_cols = nullptr;   // top-k epilogue outputs [max_rows, 512] (allocated with dense_out's arena)
   float* topk_scores = nullptr;
   size_t topk_cap = 0;
+  // ranking evaluation workspace (ocf_rank.cuh; allocated with dense_out's arena): [max_entries] each
+  uint32_t* rank_key = nullptr;
+  int32_t *rank_col = nullptr, *rank_ent = nullptr, *rank_cnt = nullptr, *rank_out = nullptr;
+  int32_t* rank_nrel = nullptr;   //   [max_rows]
+  unsigned long long* rank_ncand = nullptr;
+  bool rank_ok = false;
   int* col_state = nullptr;       // batch-side K4a: [2][n_cols] per-column count / code OR, zeroed per step
   int2* col_info = nullptr;       //   [n_cols] (first match, matches)
   uint32_t* col_bits = nullptr;   //   presence bitmap [n_cols][ceil(max_rows / 32)]
@@ -1139,6 +1146,7 @@ static int alloc_workspace(ocf_model* m, int max_rows, int64_t max_entries) {
   m->dense_mem.release();
   m->dense_out = nullptr;
   m->topk_cols = nullptr; m->topk_scores = nullptr; m->topk_cap = 0;
+  m->rank_ok = false;
   m->cfg.max_rows = max_rows;
   m->cfg.max_entries = max_entries;
   m->max_items = max_items_for(max_rows, max_entries);
@@ -2381,6 +2389,19 @@ static int ocf_score_impl(ocf_model* m, ocf_batch* b, float* out, int out_is_dev
   return OCF_OK;
 }
 
+// The full-catalogue scores of the batch into dense_out (they stay in HBM), the row's input columns set
+// to -inf when `exclude_inputs`: what the serving epilogues (top-k, ranking evaluation) read.
+static int score_to_dense(ocf_model* m, ocf_batch* b, int exclude_inputs, void* stream_) {
+  cudaStream_t st = as_stream(stream_);
+  OCF_TRY(ensure_dense(m));
+  OCF_TRY(ocf_score(m, b, m->dense_out, 1, stream_));
+  if (exclude_inputs && b->dev.n_items > 0) {
+    k_exclude_inputs<<<b->dev.n_items, 128, 0, st>>>(b->dev, m->dense_out, (long long)m->cfg.n_cols);
+    OCF_LAUNCHED();
+  }
+  return OCF_OK;
+}
+
 static int ocf_score_topk_impl(ocf_model* m, ocf_batch* b, int32_t k, int exclude_inputs, int32_t* out_cols, float* out_scores,
                               void* stream_);
 extern "C" int ocf_score_topk(ocf_model* m, ocf_batch* b, int32_t k, int exclude_inputs, int32_t* out_cols, float* out_scores,
@@ -2403,17 +2424,74 @@ static int ocf_score_topk_impl(ocf_model* m, ocf_batch* b, int32_t k, int exclud
     OCF_TRY(m->dense_mem.get(&m->topk_scores, (size_t)m->cfg.max_rows * TOPK_MAX));
     m->topk_cap = (size_t)m->cfg.max_rows * TOPK_MAX;
   }
-  OCF_TRY(ocf_score(m, b, m->dense_out, 1, stream_));          // full scores stay in HBM
-  if (exclude_inputs && b->dev.n_items > 0) {
-    k_exclude_inputs<<<b->dev.n_items, 128, 0, st>>>(b->dev, m->dense_out, (long long)m->cfg.n_cols);
-    OCF_LAUNCHED();
-  }
+  OCF_TRY(score_to_dense(m, b, exclude_inputs, stream_));
   g_prof.begin(6, st);
   k_topk<<<B, TOPK_THREADS, 0, st>>>(m->dense_out, (long long)m->cfg.n_cols, m->cfg.n_cols, k, m->topk_cols, m->topk_scores);
   OCF_LAUNCHED();
   g_prof.end(6, st);
   OCF_CUDA(cudaMemcpyAsync(out_cols, m->topk_cols, sizeof(int32_t) * (size_t)B * k, cudaMemcpyDeviceToHost, st));
   OCF_CUDA(cudaMemcpyAsync(out_scores, m->topk_scores, sizeof(float) * (size_t)B * k, cudaMemcpyDeviceToHost, st));
+  OCF_CUDA(cudaStreamSynchronize(st));
+  return OCF_OK;
+}
+
+static int ocf_rank_targets_impl(ocf_model* m, ocf_batch* b, int exclude_inputs, float min_value, int32_t* out_col,
+                                 int32_t* out_rank, int32_t* out_row_ptr, int64_t* out_n_cand, void* stream_);
+extern "C" int ocf_rank_targets(ocf_model* m, ocf_batch* b, int exclude_inputs, float min_value, int32_t* out_col,
+                                int32_t* out_rank, int32_t* out_row_ptr, int64_t* out_n_cand, void* stream_) {
+  if (b) OCF_TRY(batch_acquire(b, as_stream(stream_)));
+  const int rc = ocf_rank_targets_impl(m, b, exclude_inputs, min_value, out_col, out_rank, out_row_ptr, out_n_cand, stream_);
+  if (b && rc == OCF_OK) OCF_TRY(batch_release(b, as_stream(stream_)));
+  return rc;
+}
+static int ocf_rank_targets_impl(ocf_model* m, ocf_batch* b, int exclude_inputs, float min_value, int32_t* out_col,
+                                 int32_t* out_rank, int32_t* out_row_ptr, int64_t* out_n_cand, void* stream_) {
+  OCF_TRY(check_step(m, b, false));
+  OCF_REQUIRE(out_col && out_rank && out_row_ptr && out_n_cand, "ocf_rank_targets: null output");
+  OCF_REQUIRE(!m->cfg.sharded && m->par_mode != OCF_PAR_COLUMNS,
+              "ocf_rank_targets: a column shard holds part of the catalogue; ranks need every column");
+  cudaStream_t st = as_stream(stream_);
+  const int B = b->dev.B, E = b->dev.n_entries;
+  OCF_TRY(ensure_dense(m));
+  if (!m->rank_ok) {
+    const size_t cap = (size_t)std::max<int64_t>(m->cfg.max_entries, 1);
+    OCF_TRY(m->dense_mem.get(&m->rank_key, cap));
+    OCF_TRY(m->dense_mem.get(&m->rank_col, cap));
+    OCF_TRY(m->dense_mem.get(&m->rank_ent, cap));
+    OCF_TRY(m->dense_mem.get(&m->rank_cnt, cap));
+    OCF_TRY(m->dense_mem.get(&m->rank_out, cap));
+    OCF_TRY(m->dense_mem.get(&m->rank_nrel, (size_t)m->cfg.max_rows));
+    OCF_TRY(m->dense_mem.get(&m->rank_ncand, (size_t)m->cfg.max_rows));
+    m->rank_ok = true;
+  }
+  OCF_TRY(score_to_dense(m, b, exclude_inputs, stream_));
+  RankArgs ra{};
+  ra.bt = b->dev; ra.scores = m->dense_out; ra.ldo = m->cfg.n_cols; ra.n_cols = m->cfg.n_cols; ra.min_value = min_value;
+  ra.key = m->rank_key; ra.col = m->rank_col; ra.ent = m->rank_ent; ra.cnt = m->rank_cnt;
+  ra.n_rel = m->rank_nrel; ra.n_cand = m->rank_ncand; ra.rank = m->rank_out;
+  // enough column slices that even a batch of one row spreads over every SM, none shorter than 4096 columns
+  const int N = m->cfg.n_cols;
+  const int want = (16 * m->sm_count + B - 1) / B;
+  const int slices = std::max(1, std::min(want, (N + 4095) / 4096));
+  ra.slice_len = (int)align_up((size_t)((N + slices - 1) / slices), 4);
+  const int grid_x = (N + ra.slice_len - 1) / ra.slice_len;
+  if (B > 0) {
+    g_prof.begin(9, st);
+    k_rank_prep<<<B, RANK_THREADS, 0, st>>>(ra);
+    OCF_LAUNCHED();
+    k_rank_count<<<dim3(grid_x, B), RANK_THREADS, 0, st>>>(ra);
+    OCF_LAUNCHED();
+    k_rank_finish<<<B, RANK_THREADS, 0, st>>>(ra);
+    OCF_LAUNCHED();
+    g_prof.end(9, st);
+  }
+  static_assert(sizeof(unsigned long long) == sizeof(int64_t), "n_cand is copied as int64");
+  if (E > 0) {
+    OCF_CUDA(cudaMemcpyAsync(out_col, b->dev.ent_col, sizeof(int32_t) * (size_t)E, cudaMemcpyDeviceToHost, st));
+    OCF_CUDA(cudaMemcpyAsync(out_rank, m->rank_out, sizeof(int32_t) * (size_t)E, cudaMemcpyDeviceToHost, st));
+  }
+  OCF_CUDA(cudaMemcpyAsync(out_row_ptr, b->dev.ent_off, sizeof(int32_t) * (size_t)(B + 1), cudaMemcpyDeviceToHost, st));
+  if (B > 0) OCF_CUDA(cudaMemcpyAsync(out_n_cand, m->rank_ncand, sizeof(int64_t) * (size_t)B, cudaMemcpyDeviceToHost, st));
   OCF_CUDA(cudaStreamSynchronize(st));
   return OCF_OK;
 }

@@ -60,7 +60,8 @@ __device__ __forceinline__ void find_bin(const int* __restrict__ hist, int nb, i
 }
 
 // Bitonic sort of n (a power of two) (key, col) slots in shared memory: key descending, column ascending.
-__device__ __forceinline__ void bitonic_desc(uint32_t* key, int32_t* col, int n, bool with_col) {
+// `payload` (optional) moves with its slot.
+__device__ __forceinline__ void bitonic_desc(uint32_t* key, int32_t* col, int n, bool with_col, int32_t* payload = nullptr) {
   for (int size = 2; size <= n; size <<= 1) {
     for (int stride = size >> 1; stride > 0; stride >>= 1) {
       for (int t = threadIdx.x; t < n / 2; t += TOPK_THREADS) {
@@ -69,7 +70,11 @@ __device__ __forceinline__ void bitonic_desc(uint32_t* key, int32_t* col, int n,
         const uint32_t ka = key[lo], kb = key[hi];
         const int32_t ca = with_col ? col[lo] : 0, cb = with_col ? col[hi] : 0;
         const bool a_first = ka > kb || (ka == kb && ca < cb);
-        if (a_first != up) { key[lo] = kb; key[hi] = ka; if (with_col) { col[lo] = cb; col[hi] = ca; } }
+        if (a_first != up) {
+          key[lo] = kb; key[hi] = ka;
+          if (with_col) { col[lo] = cb; col[hi] = ca; }
+          if (payload) { const int32_t p = payload[lo]; payload[lo] = payload[hi]; payload[hi] = p; }
+        }
       }
       __syncthreads();
     }

@@ -325,6 +325,58 @@ class OmniNet(object):
             cols[cols >= 0] += self.owner.col_lo
         return cols, scores
 
+    def rank_targets(self, batch, exclude_seen=True, min_value=None):
+        """Exact rank of every relevant target of every batch row among the row's candidate columns, on
+        the device (`ocf_rank_targets`): 1-based, in the order `recommend` uses (score descending, ties by
+        lower column), so rank(t) <= k exactly when t is in `recommend(batch, k)` at position rank(t) - 1.
+        Relevant targets: the row's target columns (a repeated column once), with a stored value
+        >= `min_value` when given, minus the columns `exclude_seen` removes from the candidates (the row's
+        inputs). With pass-through split batches every target is also an input, so with `exclude_seen`
+        no row has a relevant target.
+        Returns (row_ptr int64 [rows + 1], cols int32, ranks int32, n_cand int64 [rows]): row r's relevant
+        targets are cols[row_ptr[r]:row_ptr[r + 1]] in entry order; n_cand[r] counts its candidates."""
+        if self.owner.sharded or self.comm is not None or (self.native is not None and self.native[1] == _lib.PAR_COLUMNS):
+            raise ValueError("rank_targets needs the whole catalogue; a column shard holds only part of it")
+        h = self._ensure(batch.n_rows, batch.n_entries, batch.aux_type, batch.reader)
+        dev = batch.upload(self.stream)
+        info = (C.c_int64 * 5)()
+        _lib.check(_lib.lib().ocf_batch_info(dev.handle, info))
+        rows, entries = int(info[0]), int(info[1])
+        col = np.empty(entries, dtype=np.int32)
+        rank = np.empty(entries, dtype=np.int32)
+        ent_ptr = np.empty(rows + 1, dtype=np.int32)
+        n_cand = np.empty(rows, dtype=np.int64)
+        mv = -np.inf if min_value is None else float(min_value)
+        _lib.check(_lib.lib().ocf_rank_targets(h, dev.handle, int(bool(exclude_seen)), mv, _lib.ptr(col),
+                                               _lib.ptr(rank), _lib.ptr(ent_ptr), _lib.ptr(n_cand), self.stream))
+        keep = rank > 0
+        before = np.concatenate(([0], np.cumsum(keep, dtype=np.int64)))
+        row_ptr = before[ent_ptr.astype(np.int64)]
+        return row_ptr, col[keep], rank[keep], n_cand
+
+    def evaluate_ranking(self, generator, steps, ks=(10,), exclude_seen=True, min_value=None, workers=1):
+        """Ranking quality of `recommend` over `steps` batches of `generator` (drawn as `evaluate_generator`
+        draws them, through the Prefetcher when `workers`): for every relevant target its exact rank
+        (`rank_targets`), then HR@k, precision@k, recall@k, NDCG@k for every k in `ks`, MRR and AUC, each the
+        float64 mean over the rows that have a relevant target (AUC: and at least one other candidate).
+        See `ranking` for the definitions. Returns a dict with those means and "rows" / "AUC_rows", the
+        number of rows behind them. Draws nothing from np.random beyond what the generator draws; leaves
+        the weights, the optimizer state and the metric log as they were."""
+        from . import ranking
+        from .data_reader import Prefetcher
+        if self.owner.sharded or self.comm is not None or (self.native is not None and self.native[1] == _lib.PAR_COLUMNS):
+            raise ValueError("evaluate_ranking needs the whole catalogue; a column shard holds only part of it")
+        ks = [int(k) for k in ks]
+        steps = max(int(steps), 0)
+        sums = ranking.empty_sums(ks)
+        source = Prefetcher(generator, steps) if workers else (next(generator) for _ in range(steps))
+        for batch in source:
+            if batch is None:
+                raise RuntimeError("generator ran out of batches (it yields None after floor(n/B) batches)")
+            row_ptr, _, ranks, n_cand = self.rank_targets(batch, exclude_seen=exclude_seen, min_value=min_value)
+            ranking.accumulate(sums, ranking.metrics_from_ranks(row_ptr, ranks, n_cand, ks))
+        return ranking.finalize(sums)
+
     def _shard_encode(self, h, dev, batch):
         """Column shards: encoder partial sums + their all-reduce before predict/score (this
         rank's output then holds its own columns)."""

@@ -78,13 +78,19 @@ def compute_full_RMSE(predictions, targets, ratings_count):
 
 def run(config: TrainConfig, reader: Optional[DataReader] = None, metadata: Optional[dict] = None,
         rating_range: Optional[float] = None, save_models: bool = True, verbose: int = 1,
-        reference_first_epoch_fallback: bool = False) -> dict:
+        reference_first_epoch_fallback: bool = False, ranking_ks: Optional[List[int]] = None,
+        ranking_min_value: Optional[float] = None) -> dict:
     """The body of `train.py`. Returns a dict with the history, the best epoch and test results.
 
     `reference_first_epoch_fallback`: the reference never saves epoch 1 (train.py:164-165), so when epoch 1 stays
     the best its reload of "the best model" fails and it tests the LIVE model, i.e. the last epoch's weights
     (train.py:194-197). False (default) tests epoch 1's weights, which is what the script means to do; True
-    reproduces what it does."""
+    reproduces what it does.
+
+    `ranking_ks`: also rank the test targets against the full catalogue (`OmniNet.evaluate_ranking`, seen items
+    excluded, targets with a value below `ranking_min_value` not relevant) and report HR / precision / recall /
+    NDCG at every k, MRR and AUC in results["test_ranking"] (ablation: one entry per test sparsity). It runs after
+    every test procedure of the script, so the other results and their NumPy stream are those of a run without it."""
     c = config
     if c.useTimestamps or c.use_sparse_representation or c.use_experimental_sparse_masking_layer:
         raise NotImplementedError("timestamps / sparse representation / experimental masking layer are out of scope")
@@ -200,5 +206,17 @@ def run(config: TrainConfig, reader: Optional[DataReader] = None, metadata: Opti
         rmse = float(np.sqrt(sse / ratings_count)) if ratings_count else float("nan")
         print("Manual test RMSE is ", rmse)
         results["manual_test_rmse"] = rmse
+    if ranking_ks is not None:
+        print("\nEvaluating ranking of the test targets")
+        if c.eval_mode == "ablation":
+            results["test_ranking"] = {}
+            for test_sparsity in c.test_sparsities:
+                results["test_ranking"][test_sparsity] = m.evaluate_ranking(
+                    gen("test", test_sparsity), test_steps, ks=ranking_ks, min_value=ranking_min_value)
+        else:
+            results["test_ranking"] = m.evaluate_ranking(gen("test", None), test_steps, ks=ranking_ks,
+                                                         min_value=ranking_min_value)
+        if verbose:
+            print("Test ranking: ", results["test_ranking"])
     return results
 
